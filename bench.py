@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- masked-NST image-steps/s @640x400 VGG-19 (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: a closure evaluation (VGG-19 forward to the deepest tap,
 style + content losses, backward to the image) plus one L-BFGS iteration for every image of the batch.
@@ -133,7 +133,7 @@ class ClockSampler:
 # ---------------------------------------------------------------------------------------------------------------
 # CPU arm: the reference path's CPU implementation (oracle port)
 # ---------------------------------------------------------------------------------------------------------------
-def cpu_reference_rate(steps, warmup, threads=None):
+def cpu_reference_rate(steps, warmup, threads=None, dump_dir=None):
     """B = 1 closure evaluations + L-BFGS on one 640x400 masked eye (BASELINE config[0] shape), all host threads.
     The forward runs the WHOLE vgg19.features stack to pool5 like the reference does (models/vgg/vgg.py:87),
     although nothing past relu4_2 is consumed.  Returns image-steps/s."""
@@ -153,10 +153,16 @@ def cpu_reference_rate(steps, warmup, threads=None):
     opt = O.LBFGS(x, lr=1.0)
     count = [0]
     t0 = [None]
+    total = warmup + steps
+
+    class Done(Exception):
+        """Raised by the closure after the last timed evaluation: opt.step() runs up to 20 of them per call."""
 
     def closure():
         if count[0] == warmup:
             t0[0] = time.perf_counter()
+        if count[0] == total:
+            raise Done
         with torch.no_grad():
             x.clamp_(0, 1)
         xv = x.detach().requires_grad_(True)
@@ -169,12 +175,15 @@ def cpu_reference_rate(steps, warmup, threads=None):
         count[0] += 1
         return float(loss), g.reshape(-1)
 
-    total = warmup + steps
-    while count[0] < total:
-        opt.step(closure)
+    try:
+        while True:
+            opt.step(closure)
+    except Done:
+        pass
     dt = time.perf_counter() - t0[0]
-    done = count[0] - warmup
-    return done / dt, done, dt, threads
+    if dump_dir:   # the image an nst() caller would receive after the last timed evaluation's update
+        dump_outputs(dump_dir, {"x": x.clamp(0, 1)})
+    return steps / dt, steps, dt, threads
 
 
 def run_reference(args, rank):
@@ -198,7 +207,7 @@ def run_reference(args, rank):
               flush=True)
         return
     steps = max(1, args.steps)
-    rate, done, dt, threads = cpu_reference_rate(steps, args.warmup)
+    rate, done, dt, threads = cpu_reference_rate(steps, args.warmup, dump_dir=args.dump_outputs)
     line = {
         "impl": "reference", "metric": METRIC, "value": rate, "unit": UNIT, "n_gpus": args.gpus, "steps": done,
         "warmup": args.warmup, "ms_per_step": 1e3 * dt / done, "higher_is_better": True, "scaling": "weak",
@@ -355,6 +364,19 @@ def nst_leg(args, dev, vgg, c_dev, s_dev, BN_loss, independent, K, Wm, world, ra
         lib.isx_prof_enable(0)
         clocks = sampler.stop() if rank == 0 else None
         pairs1 = torch.cat([j.history_counts() for j in subjobs])
+        if args.dump_outputs and rank == 0:
+            # what nst() hands back after the last timed step: the images clamped to [0, 1] and each problem's losses
+            # (a problem that stopped early keeps its own last logged losses, as in NstJob.finish)
+            x, idx = dump_sample(torch.cat([j.x for j in subjobs]).clamp(0, 1), DUMP_BUDGET - (1 << 20))
+            c_loss, s_loss = [], []
+            for j in subjobs:
+                e = j.evals_done().to(j.hist_c.device).long()      # 0 while a problem still runs
+                rows = torch.where(e > 0, e - 1, j.ticks - 1)
+                cols = torch.arange(j.P, device=rows.device)
+                c_loss.append(j.hist_c[rows, cols])
+                s_loss.append(j.hist_s[rows, cols])
+            dump_outputs(args.dump_outputs, {"x": x, "x_image_index": idx.double(), "c_loss": torch.cat(c_loss),
+                                             "s_loss": torch.cat(s_loss)})
         moved = float((torch.cat([j.x for j in subjobs]) - x0).abs().mean())
         loss_first = float(sum(j.hist_s[0].sum() for j in subjobs))
         loss_last = float(sum(j.hist_s[j.ticks - 1].sum() for j in subjobs))
@@ -372,9 +394,10 @@ def nst_leg(args, dev, vgg, c_dev, s_dev, BN_loss, independent, K, Wm, world, ra
                 prefill=prefill)
 
 
-def feature_leg(dev, vgg, taps5, n_per_gpu, world, batch=32):
+def feature_leg(dev, vgg, taps5, n_per_gpu, world, batch=32, passes=1, dump_dir=None):
     """BASELINE config[2]: style features (mean/std + Gram upper triangles of the style taps) of synthetic eyes for the
-    iris classifier, image list sharded contiguously over the ranks, rows exchanged over NVLink (sharding.PeerRows)."""
+    iris classifier, image list sharded contiguously over the ranks, rows exchanged over NVLink (sharding.PeerRows).
+    `passes` timed passes over the image list; `dump_dir`: the rows of the last one (rank 0)."""
     import torch
     import torch.distributed as dist
 
@@ -414,14 +437,18 @@ def feature_leg(dev, vgg, taps5, n_per_gpu, world, batch=32):
     barrier()
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     f0.record()
-    rows = features.extract_features_sharded(vgg_feat, imgs, batch=batch, device=dev)
+    for _ in range(passes):
+        rows = features.extract_features_sharded(vgg_feat, imgs, batch=batch, device=dev)
     f1.record()
     barrier()
+    if dump_dir and (world == 1 or dist.get_rank() == 0):
+        r, idx = dump_sample(rows, DUMP_BUDGET - (1 << 20))
+        dump_outputs(dump_dir, {"rows": r, "row_index": idx.double()})
     tf = torch.tensor([f0.elapsed_time(f1)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tf, op=dist.ReduceOp.MAX)
     fl = 193.82e9 if taps5 else 131.96e9
-    rate = n_total / (float(tf.item()) / 1e3)
+    rate = passes * n_total / (float(tf.item()) / 1e3)
     out = {"metric": "Gram-feature images/sec @640x400 (%s: mean/std + Gram upper triangles)" % ("relu1_1..relu5_1" if taps5 else "relu1_1..relu4_1"),
            "value": rate, "unit": "images/s", "n_images": n_total, "feature_dim": int(rows.shape[1]),
            "all_gather_bytes": int(rows.numel() * 4), "flops_per_image": fl,
@@ -430,6 +457,39 @@ def feature_leg(dev, vgg, taps5, n_per_gpu, world, batch=32):
     del rows
     torch.cuda.empty_cache()
     return out
+
+
+DUMP_BUDGET = 64 << 20
+
+
+def dump_sample(t, budget, seed=0):
+    """(rows, row_index) of a (N, ...) tensor within `budget` bytes: all of it, else a seeded subset of rows, so that two
+    builds run with the same arguments dump the same rows."""
+    import torch
+
+    t = t.detach().cpu()
+    n = t.shape[0]
+    per_row = max(1, t[:1].numel() * t.element_size())
+    keep = min(n, max(1, budget // per_row))
+    idx = torch.arange(n) if keep == n else torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+    return t[idx], idx
+
+
+def dump_outputs(d, arrays):
+    """Write {name: tensor} as d/<name>.npy in float32 (float64 stays float64); the total must fit DUMP_BUDGET."""
+    import numpy as np
+    import torch
+
+    os.makedirs(d, exist_ok=True)
+    out = {}
+    for name, t in arrays.items():
+        t = torch.as_tensor(t).detach().cpu()
+        out[name] = t.numpy() if t.dtype == torch.float64 else t.float().numpy()
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BUDGET:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_BUDGET))
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -512,6 +572,8 @@ def landmarks_leg(args, dev, lib, world, rank, local):
         g = net(seg)
         e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"gaze": g})
     launches = int(lib.isx_launch_count() - launches0)
     prof = (ctypes.c_double * 12)()
     _lib.call("isx_prof_collect", prof, 12)
@@ -593,7 +655,12 @@ def main():
     ap.add_argument("--feature-batch", type=int, default=64, help="images per forward pass of the feature-extraction leg")
     ap.add_argument("--opt", action="append", default=[], help="name=value: libisx kernel-selection option (isx_set_option), repeatable")
     ap.add_argument("--e2e-evals", type=int, default=300, help="evaluations of the end-to-end job (BASELINE config[1]: 300)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (at most 64 MB, "
+                         "a seeded sample of the images or rows when larger) to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference" and args.config == "landmarks":
+        raise SystemExit("--dump-outputs: the landmarks reference arm times cv2 calls and keeps none of their results")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -602,8 +669,8 @@ def main():
             args.steps = 40
         run_reference(args, rank)
         return
-    if args.steps is None:
-        args.steps = 100
+    if args.steps is None:   # a step: one tick of an NST job, one pass over the feature images, one batch of frames
+        args.steps = {"feat4": 1, "feat5": 1, "frames2020": 2}.get(args.config, 100)
     if args.warmup < 3:
         args.warmup = 3
 
@@ -640,9 +707,10 @@ def main():
 
     # ------------------------------------------------------------------ feature-only configs
     if cfgname in ("feat4", "feat5"):
-        feat = feature_leg(dev, vgg, cfgname == "feat5", args.feature_images, world, batch=args.feature_batch)
+        feat = feature_leg(dev, vgg, cfgname == "feat5", args.feature_images, world, batch=args.feature_batch, passes=K,
+                           dump_dir=args.dump_outputs)
         if rank == 0:
-            line = {"metric": feat["metric"], "value": feat["value"], "unit": "images/s", "n_gpus": world, "steps": 1,
+            line = {"metric": feat["metric"], "value": feat["value"], "unit": "images/s", "n_gpus": world, "steps": K,
                     "warmup": 1, "ms_per_step": 1e3 * feat["n_images"] / feat["value"], "higher_is_better": True,
                     "scaling": "weak", "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
                     "config": {"workload": "BASELINE config[2]: %d synthetic 640x400 eyes per GPU -> style features, sharded, "
@@ -659,7 +727,12 @@ def main():
     if cfgname == "frames2020":
         from iris_b200 import frames as frames_mod
 
-        line = frames_mod.bench_frames2020(args, dev, vgg, world, rank)
+        def dump_frames(frames):
+            f, idx = dump_sample(frames, DUMP_BUDGET - (1 << 20))
+            dump_outputs(args.dump_outputs, {"frames": f, "frame_index": idx.double()})
+
+        line = frames_mod.bench_frames2020(args, dev, vgg, world, rank,
+                                           dump=dump_frames if args.dump_outputs and rank == 0 else None)
         if rank == 0:
             print(json.dumps(line), flush=True)
         finish()

@@ -106,11 +106,12 @@ def stylize_frames(frames: torch.Tensor,
 # ---------------------------------------------------------------------------------------------------------------
 # BASELINE config[3]: OpenEDS2020-shaped synthetic eye sequences, privacy-masking NST, sharded over the GPUs of a box
 # ---------------------------------------------------------------------------------------------------------------
-def bench_frames2020(args, dev, vgg, world: int, rank: int):
+def bench_frames2020(args, dev, vgg, world: int, rank: int, dump=None):
     """One JSON line for `bench.py --config frames2020`: every rank stylises its own batches of 128 synthetic 400x640
     frames (the 2020 driver's batch size, …2020.py:211) against ONE fixed 224x224 style iris (…2020.py:238-249), default
     StyleLoss_BN, the batch as one L-BFGS problem, 200 evaluations, from pinned host frames + label maps to pinned host
-    frames -- mask, bbox, crop, resize, NST, composite all inside the timed region."""
+    frames -- mask, bbox, crop, resize, NST, composite all inside the timed region.  One step = one batch (`--steps`).
+    `dump(frames)`, if given, receives the stylised frames of the last batch (pinned host memory)."""
     import time
 
     import numpy as np
@@ -120,7 +121,7 @@ def bench_frames2020(args, dev, vgg, world: int, rank: int):
 
     Hf, Wf = 400, 640                                   # OpenEDS2020 frames are (1,400,640) (gaze_estimators.py:121)
     B = args.batch or 128
-    n_batches = 2
+    n_batches = args.steps
     epochs = 200
     fr, sg = synthetic.synthetic_batch([50000 * rank + i for i in range(B)], Hf, Wf)
     frames_h = torch.from_numpy(fr).pin_memory()
@@ -151,6 +152,8 @@ def bench_frames2020(args, dev, vgg, world: int, rank: int):
         evals = info["evals"]
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
+    if dump is not None:
+        dump(out_h)
     t = torch.tensor([dt], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
