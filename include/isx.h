@@ -381,17 +381,17 @@ int isx_angular_distance(const float* v1, const float* v2, int n, int d, float* 
  * launching stream; after a device sync isx_prof_collect fills out[3*family + {0,1,2}] = {launches, total ms,
  * total algorithmic work (FLOPs for 0/1, bytes for 2/3)}; n_out >= 12. */
 unsigned long long isx_launch_count(void);
-/* kernel-selection knobs (tests, experiments; defaults in parentheses): "c64" (1) resident-weight kernel for the 64->64
- * layers, "halo2" (1) halo-patch pair kernel for the mid layers, "tail_n" (1) taps-in-N image-gradient tail -- 0 sends
- * the call to the generic kernel, 2 ("c64", "halo2") forces the kernel on every applicable call; "c64_slots",
- * "halo2_stages": ring depths (0 = as many as fit); "smem_reserve_kb" (0): shared memory per SM the persistent conv CTAs leave
- * free (<= 22) so that one TMEM-free streaming CTA of another stream -- the L-BFGS history passes -- can be resident beside
- * them; "pool_idx" (1): the NST driver routes the max-pool + ReLU backward through the index bytes the fused conv epilogues
- * emit and does not store untapped pre-pool activations (0: stores them and re-reads them in the backward); "head_ctas" (5):
- * resident CTAs per SM the conv1_1 head is compiled for (5 or 8); "sweep64" (1): tap-stacked sweep kernel for
- * the 64 -> 64 layers (conv_sweep.cu; 0 never, 1 the forward launches whose 128-pixel strips fit the image, 2 every applicable
- * call), "sweep_dbg": its diagnostics; "lm_planes" (0): experiment knob of the landmark bit-plane kernel (requests in flight per
- * warp + 100 x grid size in halves of a resident wave).  Unknown names return non-zero. */
+/* kernel-selection options (defaults in parentheses).  The first four choose among kernels for the same convolution;
+ * the default 1 picks one from the shapes of the call, 0 sends the call to the generic kernel, 2 forces the kernel on every
+ * applicable call (tests compare each kernel with the generic one this way):
+ *   "c64" (1): resident-weight kernel for the 64 -> 64 layers;
+ *   "halo2" (1): halo-patch pair kernel for the mid layers;
+ *   "tail_n" (1): taps-in-N image-gradient tail (0 or 1);
+ *   "sweep64" (1): tap-stacked sweep kernel for the 64 -> 64 layers (conv_sweep.cu; 1: the forward launches whose 128-pixel
+ *     strips fit the image).
+ * "smem_reserve_kb" (0): shared memory per SM the persistent conv CTAs leave free (<= 22), so that one TMEM-free streaming CTA
+ * of another stream -- the L-BFGS history passes -- can be resident beside them.
+ * Unknown names return non-zero. */
 int isx_set_option(const char* name, int value);   /* on the calling thread's current context */
 int isx_get_option(const char* name, int* value);
 int isx_prof_enable(int on);

@@ -39,10 +39,6 @@ def load():
         if hasattr(lib, name):
             getattr(lib, name).restype = ctypes.c_int64
     _lib = lib
-    # kernel-selection knobs from the environment (ISX_C64=0, ISX_HALO2=2, ISX_TAIL_N=0) -> isx_set_option
-    for env, opt in (("ISX_C64", "c64"), ("ISX_HALO2", "halo2"), ("ISX_TAIL_N", "tail_n")):
-        if os.environ.get(env):
-            lib.isx_set_option(opt.encode(), int(os.environ[env]))
     return lib
 
 

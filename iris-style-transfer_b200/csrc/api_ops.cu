@@ -267,35 +267,35 @@ extern "C" int isx_tap_add_mask(const isx_bf16* g, const isx_bf16* add, const fl
   return tap_add_mask(P(g), P(add), aff_a, aff_b, P(act), P(out), B, HW, C, S(stream));
 }
 
+// the option names of isx_set_option / isx_get_option and the context fields they address; nullptr: unknown name
+static int IsxContext::*option_field(const char* name) {
+  static const struct {
+    const char* name;
+    int IsxContext::*field;
+  } kOptions[] = {
+      {"c64", &IsxContext::opt_c64},
+      {"halo2", &IsxContext::opt_halo2},
+      {"tail_n", &IsxContext::opt_tail_n},
+      {"sweep64", &IsxContext::opt_sweep64},
+      {"smem_reserve_kb", &IsxContext::opt_smem_reserve_kb},
+  };
+  for (const auto& o : kOptions)
+    if (strcmp(name, o.name) == 0) return o.field;
+  return nullptr;
+}
+
 extern "C" int isx_set_option(const char* name, int value) {
   ISX_REQUIRE(name != nullptr, "isx_set_option: null name");
-  if (strcmp(name, "c64") == 0) { isx_ctx()->opt_c64 = value; return 0; }
-  if (strcmp(name, "tail_n") == 0) { isx_ctx()->opt_tail_n = value; return 0; }
-  if (strcmp(name, "halo2") == 0) { isx_ctx()->opt_halo2 = value; return 0; }
-  if (strcmp(name, "halo2_stages") == 0) { isx_ctx()->opt_halo2_stages = value; return 0; }
-  if (strcmp(name, "c64_slots") == 0) { isx_ctx()->opt_c64_slots = value; return 0; }
-  if (strcmp(name, "smem_reserve_kb") == 0) { isx_ctx()->opt_smem_reserve_kb = value; return 0; }
-  if (strcmp(name, "head_ctas") == 0) { isx_ctx()->opt_head_ctas = value; return 0; }
-  if (strcmp(name, "sweep64") == 0) { isx_ctx()->opt_sweep64 = value; return 0; }
-  if (strcmp(name, "sweep_dbg") == 0) { isx_ctx()->opt_sweep_dbg = value; return 0; }
-  if (strcmp(name, "pool_idx") == 0) { isx_ctx()->opt_pool_idx = value; return 0; }
-  if (strcmp(name, "lm_planes") == 0) { isx_ctx()->opt_lm_planes = value; return 0; }
-  ISX_REQUIRE(false, "isx_set_option: unknown option '%s'", name);
+  int IsxContext::*field = option_field(name);
+  ISX_REQUIRE(field != nullptr, "isx_set_option: unknown option '%s'", name);
+  isx_ctx()->*field = value;
+  return 0;
 }
 
 extern "C" int isx_get_option(const char* name, int* value) {
   ISX_REQUIRE(name != nullptr && value != nullptr, "isx_get_option: null pointer");
-  const IsxContext* c = isx_ctx();
-  if (strcmp(name, "c64") == 0) { *value = c->opt_c64; return 0; }
-  if (strcmp(name, "tail_n") == 0) { *value = c->opt_tail_n; return 0; }
-  if (strcmp(name, "halo2") == 0) { *value = c->opt_halo2; return 0; }
-  if (strcmp(name, "halo2_stages") == 0) { *value = c->opt_halo2_stages; return 0; }
-  if (strcmp(name, "c64_slots") == 0) { *value = c->opt_c64_slots; return 0; }
-  if (strcmp(name, "smem_reserve_kb") == 0) { *value = c->opt_smem_reserve_kb; return 0; }
-  if (strcmp(name, "head_ctas") == 0) { *value = c->opt_head_ctas; return 0; }
-  if (strcmp(name, "sweep64") == 0) { *value = c->opt_sweep64; return 0; }
-  if (strcmp(name, "sweep_dbg") == 0) { *value = c->opt_sweep_dbg; return 0; }
-  if (strcmp(name, "pool_idx") == 0) { *value = c->opt_pool_idx; return 0; }
-  if (strcmp(name, "lm_planes") == 0) { *value = c->opt_lm_planes; return 0; }
-  ISX_REQUIRE(false, "isx_get_option: unknown option '%s'", name);
+  int IsxContext::*field = option_field(name);
+  ISX_REQUIRE(field != nullptr, "isx_get_option: unknown option '%s'", name);
+  *value = isx_ctx()->*field;
+  return 0;
 }

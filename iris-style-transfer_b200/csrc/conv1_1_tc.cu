@@ -41,8 +41,8 @@ struct C11Params {
 
 // TW (power of two, TH = 128 / TW) is a template parameter: the patch index arithmetic (i % PW, i / (PW*PH), tid % TW)
 // then compiles to multiply-shift instead of ~15 integer divisions per thread and tile.
-template <int TW, int MINB>
-__global__ void __launch_bounds__(128, MINB)
+template <int TW>
+__global__ void __launch_bounds__(128, 5)
 conv1_1_tc_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmO, const C11Params p) {
   constexpr int TH = 128 / TW;
   // Everything lives in DYNAMIC shared memory declared 1024-byte aligned (no static arrays in front of it, no alignment
@@ -239,21 +239,16 @@ int conv1_1_fwd_tc(const float* x, int xc, const float* mask, int mask_b, const 
   }
   const size_t smem_bytes = kC11Patch + 4 * 3 * (p.TW + 2) * (p.TH + 2);
   // Latency-bound kernel (per tile: patch -> smem, row build, MMA round trip, TMEM read, TMA store): what hides the chain
-  // is the number of resident CTAs.  Compiled for 8 per SM (64 registers, 28 KB of shared memory and 64 TMEM columns each;
-  // "head_ctas" = 5 selects the 93-register build that fits five).  Measured grid sweep at 640x400 (us/image, five resident):
-  // 148 x 5 12.0, x 6 15.4 (partial second wave), x 10 11.9, x 32 11.8 -> many short CTAs make the static tile split
-  // insensitive to wave quantisation.
+  // is the number of resident CTAs.  Compiled for five per SM (89-96 registers, 28 KB of shared memory and 64 TMEM columns
+  // each).  A build for eight per SM (64 registers, 40-192 B of spill stores) was measured SLOWER on a B200: 12.7 against
+  // 11.1 us/image at 640x400 -- the tile chain is bound by instruction issue and shared-memory traffic, not by occupancy.
+  // Measured grid sweep at 640x400 (us/image, five resident): 148 x 5 12.0, x 6 15.4 (partial second wave), x 10 11.9,
+  // x 32 11.8 -> many short CTAs make the static tile split insensitive to wave quantisation.
   const int grid = std::min(p.n_tiles, kNumSMs * 32);
-  const bool dense = isx_ctx()->opt_head_ctas >= 8;
 #define ISX_C11_CASE(TW_)                                                                                                   \
   case TW_:                                                                                                                 \
-    if (dense) {                                                                                                            \
-      ISX_CHECK_CUDA(cudaFuncSetAttribute(conv1_1_tc_kernel<TW_, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes)); \
-      conv1_1_tc_kernel<TW_, 8><<<grid, 128, smem_bytes, s>>>(tmW, tmO, p);                                                 \
-    } else {                                                                                                                \
-      ISX_CHECK_CUDA(cudaFuncSetAttribute(conv1_1_tc_kernel<TW_, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes)); \
-      conv1_1_tc_kernel<TW_, 5><<<grid, 128, smem_bytes, s>>>(tmW, tmO, p);                                                 \
-    }                                                                                                                       \
+    ISX_CHECK_CUDA(cudaFuncSetAttribute(conv1_1_tc_kernel<TW_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes)); \
+    conv1_1_tc_kernel<TW_><<<grid, 128, smem_bytes, s>>>(tmW, tmO, p);                                                      \
     break;
   switch (p.TW) {
     ISX_C11_CASE(128) ISX_C11_CASE(64) ISX_C11_CASE(32) ISX_C11_CASE(16) ISX_C11_CASE(8) ISX_C11_CASE(4) ISX_C11_CASE(2)

@@ -406,7 +406,7 @@ static int launch_c64(const ConvArgs& a, cudaStream_t stream) {
   p.pool_idx = p.fuse_pool ? a.pool_idx : nullptr;
   p.skip_out = (p.fuse_pool && a.pool_idx != nullptr && a.skip_out) ? 1 : 0;
   p.dx_nchw = a.dx_nchw; p.xc = a.xc; p.in_mask = a.in_mask; p.mask_b = a.mask_b;
-  int hs = isx_ctx()->opt_c64_slots > 0 ? isx_ctx()->opt_c64_slots : 4;
+  int hs = 4;
   C64Layout L = c64_layout<BN, EPI>(hs, p.use_mask, p.use_gram, p.fuse_pool);
   const int cap = (227 - std::max(0, std::min(isx_ctx()->opt_smem_reserve_kb, 22))) * 1024;  // see conv_halo.cu
   while (hs > 2 && 1024 + L.total > cap) { --hs; L = c64_layout<BN, EPI>(hs, p.use_mask, p.use_gram, p.fuse_pool); }

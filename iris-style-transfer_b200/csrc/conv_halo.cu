@@ -434,7 +434,7 @@ static int launch_halo(const ConvArgs& a, cudaStream_t stream) {
   p.fuse_pool = (a.pool_out != nullptr && a.H >= 2 && a.W >= 2) ? 1 : 0;
   p.pool_idx = p.fuse_pool ? a.pool_idx : nullptr;
   p.skip_out = (p.fuse_pool && a.pool_idx != nullptr && a.skip_out) ? 1 : 0;
-  int ws = isx_ctx()->opt_halo2_stages > 0 ? std::min(isx_ctx()->opt_halo2_stages, 8) : 6;
+  int ws = 6;
   HaloLayout L = halo_layout<BN>(ws, p.use_mask, p.fuse_pool);
   // "smem_reserve_kb" (<= 22): leave that much of the SM's shared memory free, so that one TMEM-free streaming CTA (the
   // L-BFGS passes of another stream) can be resident beside this persistent CTA and use the HBM bandwidth it leaves idle

@@ -65,7 +65,6 @@ struct SweepParams {
   const float* aff_a;
   const float* aff_b;
   uint8_t* pool_idx;
-  int dbg;             // diagnostics ("sweep_dbg"): 1 = issue no MMAs, 2 = epilogue only drains TMEM, 8 = clock64 profile of block 0
 };
 
 struct SweepLayout {
@@ -127,11 +126,11 @@ struct SweepWalk {
 // unless it wraps around the ring (S = 6, 7: two MMAs); the first step gives the new slot j = 2 its own MMA with accumulate = 0.
 // uz: a runtime value that is always zero, derived from a kernel parameter -- added to the constant TMEM addresses so that
 // they are formed on the uniform datapath (a literal goes through a vector register and an R2UR per MMA).
-template <int S, bool SMALL = false>
+template <int S>
 __device__ __forceinline__ void sweep_interior(uint32_t a_lo, uint32_t w_lo, uint32_t hi, uint32_t uz) {
-  constexpr uint32_t I64 = umma_idesc_bf16(128, SMALL ? 16 : 64, false, false);
-  constexpr uint32_t I128 = umma_idesc_bf16(128, SMALL ? 16 : 128, false, false);
-  constexpr uint32_t I192 = umma_idesc_bf16(128, SMALL ? 16 : 192, false, false);
+  constexpr uint32_t I64 = umma_idesc_bf16(128, 64, false, false);
+  constexpr uint32_t I128 = umma_idesc_bf16(128, 128, false, false);
+  constexpr uint32_t I192 = umma_idesc_bf16(128, 192, false, false);
   constexpr uint32_t J1 = 8192 >> 4, J2 = 16384 >> 4;   // weight slab of output j inside the strip-tap block
 #pragma unroll
   for (int ku = 0; ku < 3; ++ku) {
@@ -157,36 +156,6 @@ __device__ __forceinline__ void sweep_interior(uint32_t a_lo, uint32_t w_lo, uin
         umma_bf16_lohi(uz, a, hi, b + J1, hi, I128, 1u);
       }
     }
-  }
-}
-// The same with the ring slot as a runtime value: one copy of the code (the eight instantiations above take turns, strip by
-// strip, in the instruction cache), TMEM addresses and instruction descriptors computed once per strip.
-__device__ __forceinline__ void sweep_interior_rt(uint32_t a_lo, uint32_t w_lo, uint32_t hi, uint32_t S) {
-  constexpr uint32_t I64 = umma_idesc_bf16(128, 64, false, false);
-  constexpr uint32_t I128 = umma_idesc_bf16(128, 128, false, false);
-  constexpr uint32_t I192 = umma_idesc_bf16(128, 192, false, false);
-  constexpr uint32_t J1 = 8192 >> 4, J2 = 16384 >> 4;
-  const uint32_t dA = S * 64;
-  const bool split = S >= 6;                          // window wraps: second MMA at column 0
-  const uint32_t iA = S <= 5 ? I192 : (S == 6 ? I128 : I64);
-  const uint32_t iB = S == 6 ? I64 : I128, bB = S == 6 ? J2 : J1;
-  const uint32_t d2 = ((S + 2) & 7) * 64;
-  {  // step (ku = 0, k = 0): j = 0, 1 accumulate, j = 2 starts a new accumulator
-    if (S <= 6) {
-      umma_bf16_lohi(dA, a_lo, hi, w_lo, hi, I128, 1u);
-    } else {
-      umma_bf16_lohi(dA, a_lo, hi, w_lo, hi, I64, 1u);
-      umma_bf16_lohi(0, a_lo, hi, w_lo + J1, hi, I64, 1u);
-    }
-    umma_bf16_lohi(d2, a_lo, hi, w_lo + J2, hi, I64, 0u);
-  }
-#pragma unroll
-  for (int st = 1; st < 12; ++st) {
-    const int ku = st >> 2, k = st & 3;
-    const uint32_t a = a_lo + ((ku * 128 + k * 32) >> 4);
-    const uint32_t b = w_lo + ((ku * 3 * 8192 + k * 32) >> 4);
-    umma_bf16_lohi(dA, a, hi, b, hi, iA, 1u);
-    if (split) umma_bf16_lohi(0, a, hi, b + bB, hi, iB, 1u);
   }
 }
 // fused Gram backward of one output strip in ring slot S: + act . D_b (N = 64, K = 64)
@@ -269,12 +238,8 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           tma_load_2d(smem + L.w + (ku * 3 + (2 - ks)) * 8192, &tmW, w_full, 0, (ky * 3 + kx) * 64);
         }
       uint32_t ps = 0, pph = 0, as = 0, aph = 0, ds = 0, dph = 0;
-      const bool pprof = (p.dbg & 8) && blockIdx.x == 0;
-      long long pw_patch = 0, pw_act = 0, pn = 0;
       auto load_act = [&](int u0, int vo, int b) {
-        const long long t0 = pprof ? clock64() : 0;
         mbar_wait(&act_empty[as], aph ^ 1);
-        if (pprof) pw_act += clock64() - t0;
         mbar_arrive_expect_tx(&act_full[as], kSwTile);
         tma_load_4d(smem + L.act + as * kSwTile, &tmM, &act_full[as], 0, u0, vo, b);
         if (++as == 4) { as = 0; aph ^= 1; }
@@ -290,9 +255,7 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           if (ds == 0) dph ^= 1;
         }
         for (int vin = J.vin0; vin <= J.vin1; ++vin) {
-          const long long t0 = pprof ? clock64() : 0;
           mbar_wait(&patch_empty[ps], pph ^ 1);
-          if (pprof) { pw_patch += clock64() - t0; ++pn; }
           mbar_arrive_expect_tx(&patch_full[ps], kSwPatchBytes);
           tma_load_4d(smem + L.patch + ps * kSwPatch, &tmA, &patch_full[ps], 0, J.u0 - 1, vin, J.b);
           if (++ps == static_cast<uint32_t>(PS)) { ps = 0; pph ^= 1; }
@@ -302,7 +265,6 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           }
         }
       }
-      if (pprof && pn > 0) printf("sweep producer, %lld strips: patch_empty wait %lld, act_empty wait %lld cycles per strip\n", pn, pw_patch / pn, pw_act / pn);
     }
   } else if (warp == 1) {
     // ================================ MMA issuer ===========================================
@@ -328,10 +290,6 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       uint32_t g0 = 0;           // running number of the job's first output strip
       // An mbarrier probe costs 150-270 cycles even when its phase completed long ago: the probes of the NEXT strip's
       // barriers (its patch, the ring slot it touches first) are issued before this strip's MMAs and consumed afterwards.
-      long long tt[4] = {0, 0, 0, 0};
-      long long nstrips = 0, tfast = 0, nfast = 0;
-      const bool prof = (p.dbg & 8) && blockIdx.x == 0;
-      const bool no_mma = (p.dbg & 1) != 0;
       SweepWalk walk(p);
       SweepJob J;
       while (walk.next(J)) {
@@ -341,8 +299,7 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           const uint32_t gj0 = g0 + static_cast<uint32_t>(vin - 1 - J.vs);      // running number of output j = 0 (may be "-1")
           const bool first_in = vin == J.vin0;
           // steady state: eight interior strips in a row, starting ring-aligned -> straight-line code with constant slots
-          if ((gj0 & 7) == 0 && !first_in && vin - 1 >= J.vs && vin + 8 <= J.ve && (p.dbg & ~8) == 0) {
-            const long long cb = prof ? clock64() : 0;
+          if ((gj0 & 7) == 0 && !first_in && vin - 1 >= J.vs && vin + 8 <= J.ve) {
             const uint32_t q = (gj0 >> 3) & 1;
             const uint32_t d_lo = d_lo0 + ds * (8192 >> 4);
 #define ISX_SWEEP_FAST(S_)                                                                                                   \
@@ -372,19 +329,15 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             ISX_SWEEP_FAST(0); ISX_SWEEP_FAST(1); ISX_SWEEP_FAST(2); ISX_SWEEP_FAST(3);
             ISX_SWEEP_FAST(4); ISX_SWEEP_FAST(5); ISX_SWEEP_FAST(6); ISX_SWEEP_FAST(7);
 #undef ISX_SWEEP_FAST
-            if (prof) { tfast += clock64() - cb; nfast += 8; }
             vin += 7;
             continue;
           }
           const bool interior = !first_in && ja == 0 && jb == 2;
-          long long c0 = 0, c1 = 0, c2 = 0, c3 = 0;
-          if (prof) c0 = clock64();
           // first touches (in running order): everything at the first input strip of a job, afterwards only j = 2
           for (int j = first_in ? ja : 2; j <= jb; ++j) {
             const uint32_t g = gj0 + j;
             if (!(s_ready && s_probed == g)) mbar_wait(&slot_empty[g & 7], ((g >> 3) & 1) ^ 1);
           }
-          if (prof) c1 = clock64();
           if (!p_ready) mbar_wait(&patch_full[ps], pph);
           tc_fence_after();
           {
@@ -393,15 +346,7 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             s_probed = gj0 + 3;   // the slot the next strip touches first (when it is an ordinary strip)
             s_ready = mbar_try_wait(&slot_empty[s_probed & 7], ((s_probed >> 3) & 1) ^ 1);
           }
-          if (prof) c2 = clock64();
-          if (no_mma) {
-          } else if (interior && (p.dbg & 4)) {   // diagnostics: the same instruction stream with N = 16 (wrong results)
-#define ISX_SWEEP_CALL(S_) sweep_interior<S_, true>(a_lo, w_lo, hi, uz)
-            ISX_SWEEP_SWITCH(gj0 & 7, ISX_SWEEP_CALL)
-#undef ISX_SWEEP_CALL
-          } else if (interior && (p.dbg & 16)) {
-            sweep_interior_rt(a_lo, w_lo, hi, gj0 & 7);
-          } else if (interior) {
+          if (interior) {
 #define ISX_SWEEP_CALL(S_) sweep_interior<S_>(a_lo, w_lo, hi, uz)
             ISX_SWEEP_SWITCH(gj0 & 7, ISX_SWEEP_CALL)
 #undef ISX_SWEEP_CALL
@@ -435,10 +380,7 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
               }
             }
           }
-          if (prof) c3 = clock64();
           umma_commit(&patch_empty[ps]);
-          const uint32_t a_cur = a_lo;
-          (void)a_cur;
           a_lo += kSwPatch >> 4;
           if (++ps == static_cast<uint32_t>(PS)) { ps = 0; pph ^= 1; a_lo = a_lo0; }
           // outputs that are complete now: vin - 1, and vin itself at the last input strip of a run that ends at the image border
@@ -450,17 +392,12 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
               mbar_wait(&act_full[as], aph);
               tc_fence_after();
               const uint32_t a2 = act_lo0 + as * (kSwTile >> 4), b2 = d_lo0 + ds * (8192 >> 4);
-              if (!no_mma) {
 #define ISX_SWEEP_CALL(S_) sweep_gram<S_>(a2, b2, hi)
-                ISX_SWEEP_SWITCH(g & 7, ISX_SWEEP_CALL)
+              ISX_SWEEP_SWITCH(g & 7, ISX_SWEEP_CALL)
 #undef ISX_SWEEP_CALL
-              }
               if (++as == 4) { as = 0; aph ^= 1; }
             }
             umma_commit(&slot_full[g & 7]);
-          }
-          if (prof) {
-            tt[0] += c1 - c0; tt[1] += c2 - c1; tt[2] += c3 - c2; tt[3] += clock64() - c3; ++nstrips;
           }
         }
         if (p.use_gram) {
@@ -470,10 +407,6 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
         g0 += static_cast<uint32_t>(J.ve - J.vs + 1);
       }
-      if (prof && nfast > 0) printf("sweep MMA thread, fast path: %lld strips, %lld cycles per strip\n", nfast, tfast / nfast);
-      if (prof && nstrips > 0)
-        printf("sweep MMA thread, %lld strips: slot_empty wait %lld, patch_full wait + probes %lld, issue %lld, commits %lld cycles per strip\n",
-               nstrips, tt[0] / nstrips, tt[1] / nstrips, tt[2] / nstrips, tt[3] / nstrips);
     }
   } else {
     // ================================ epilogue (8 warps) ===================================
@@ -493,9 +426,6 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     uint32_t prevw[16];       // regpool: the even strip of the current pair, packed bf16x2
 #pragma unroll
     for (int e = 0; e < 16; ++e) prevw[e] = 0u;
-    long long et[6] = {0, 0, 0, 0, 0, 0};
-    long long estrips = 0;
-    const bool eprof = (p.dbg & 8) && blockIdx.x == 0 && leader;
     SweepWalk walk(p);
     SweepJob J;
     while (walk.next(J)) {
@@ -508,31 +438,17 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         const uint32_t ss = static_cast<uint32_t>(vo) & 1;   // staging slot: even / odd sweep coordinate
         const uint32_t as = at & 3;                          // dgrad: mask strip of this output, overwritten in place by the result
         uint8_t* stg = p.use_mask ? smem + L.act + as * kSwTile : smem + L.stg + ss * kSwTile;
-        long long e0 = 0, e1 = 0;
-        if (eprof) e0 = clock64();
         if (!f_ready) mbar_wait(&slot_full[slot], (g >> 3) & 1);
         tc_fence_after();
-        if (eprof) e1 = clock64();
         uint32_t v[32];
         tmem_ld_32x32(tmem_base + slot * 64 + n + (static_cast<uint32_t>(q * 32) << 16), v);
         tmem_ld_wait();
-        long long e2 = 0, e3 = 0, e4 = 0;
-        if (eprof) e2 = clock64();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&slot_empty[slot]);   // accumulator read: the ring slot goes back to the MMA warp
         f_ready = mbar_try_wait(&slot_full[(g + 1) & 7], ((g + 1) >> 3) & 1);   // consumed at the top of the next strip
         const bool m_now = m_ready;
         if (p.use_mask) m_ready = mbar_try_wait(&act_full[(at + 1) & 3], ((at + 1) >> 2) & 1);
-        if (p.dbg & 2) {
-          if (p.use_mask) {
-            mbar_wait(&act_full[as], (at >> 2) & 1);
-            asm volatile("bar.sync 1, 256;" ::: "memory");
-            if (leader) mbar_arrive(&act_empty[as]);
-            ++at;
-          }
-          continue;
-        }
         float f[32];
 #pragma unroll
         for (int e = 0; e < 32; ++e) f[e] = __uint_as_float(v[e]) + bias_r[e];
@@ -593,7 +509,6 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           if ((vo & 1) == 0) {
 #pragma unroll
             for (int e = 0; e < 16; ++e) prevw[e] = w[e];
-            if (eprof) { et[0] += e1 - e0; et[1] += clock64() - e1; ++estrips; }
             continue;
           }
           const bool odd = (lane & 1) != 0;   // this lane pools words 8..15 of its 16, the even lane of the pair words 0..7
@@ -640,7 +555,6 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             tma_store_4d(&tmP, pst, 0, J.u0 >> 1, vo >> 1, J.b);
             tma_store_commit();
           }
-          if (eprof) { et[0] += e1 - e0; et[1] += clock64() - e1; ++estrips; }
           continue;
         }
         uint8_t* rowp = stg + row * 128;
@@ -655,14 +569,12 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           *reinterpret_cast<uint4*>(rowp + chunk * 16) = o;
         }
         fence_proxy_async_smem();
-        if (eprof) e3 = clock64();
         // the other staging slot is rewritten by the next strip: the TMA stores that read it must be done with it
         if (leader) {
           tma_store_wait_read<0>();
           if (act_held != 0xffffffffu) { mbar_arrive(&act_empty[act_held]); act_held = 0xffffffffu; }   // its store has read it
         }
         asm volatile("bar.sync 1, 256;" ::: "memory");
-        if (eprof) e4 = clock64();
         if (leader && !p.skip_out) {
           tma_store_4d(&tmO, stg, 0, J.u0, vo, J.b);
           tma_store_commit();
@@ -709,17 +621,12 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             tma_store_commit();
           }
         }
-        if (eprof) { et[0] += e1 - e0; et[1] += clock64() - e1; et[2] += e2 - e1; et[3] += e3 - e2; et[4] += e4 - e3; ++estrips; }
       }
     }
     if (leader) {
       tma_store_wait_all<0>();
       if (act_held != 0xffffffffu) mbar_arrive(&act_empty[act_held]);
     }
-    if (eprof && estrips > 0)
-      printf("sweep epilogue leader, %lld strips: slot_full wait %lld, drain + math + stage + store %lld (tmem_ld %lld, probe + math + staging %lld, "
-             "store-read wait + barrier %lld) cycles per strip\n", estrips, et[0] / estrips, et[1] / estrips, et[2] / estrips, et[3] / estrips,
-             et[4] / estrips);
     tc_fence_before();
   }
   __syncthreads();
@@ -763,7 +670,6 @@ int conv_sweep(const ConvArgs& a, cudaStream_t stream) {
   while (ps > 2 && 1024 + L.total > 227 * 1024) { --ps; L = sweep_layout(ps, p.use_mask, p.use_gram, p.fuse_pool); }
   ISX_REQUIRE(1024 + L.total <= 227 * 1024, "conv_sweep: %d B of shared memory exceed 227 KB", 1024 + L.total);
   p.patch_slots = ps;
-  p.dbg = isx_ctx()->opt_sweep_dbg;
   const size_t smem_bytes = std::max<size_t>(1024 + L.total, 204 * 1024);  // nobody else of this library fits beside it
 
   // the NHWC tensors seen as (c, u, v, b): u = strip axis, v = sweep axis

@@ -479,16 +479,6 @@ static int launch_conv(const ConvArgs& a, int stages_override, cudaStream_t stre
   return 0;
 }
 
-// tuning knobs (isx_set_option)
-// Specialised Cin = 64 kernel (resident weights + halo patch, conv_c64.cu).  0: never; 1 (default): the 64 -> 64 layers
-// when there is at least one tile per SM; 2: every applicable call, including the N = 16 tail and tiny inputs (tests).
-// (isx_ctx()->opt_c64, default 1)
-
-// Halo-patch pair kernel (conv_halo.cu).  0: never; 1: layers with enough work items and little padding; 2: every
-// applicable call (tests).
-// (isx_ctx()->opt_halo2, default 1)
-
-
 int conv_tc(const ConvArgs& a_in, cudaStream_t stream) {
   ConvArgs a = a_in;
   if (a.dx_nchw != nullptr && isx_ctx()->opt_tail_n > 0 && isx_ctx()->opt_c64 < 2 && a.force_bn == 0 &&

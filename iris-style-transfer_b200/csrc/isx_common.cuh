@@ -43,17 +43,9 @@ struct IsxContext {
   int opt_c64 = 1;                   // "c64": resident-weight kernel for the 64 -> 64 layers (0 never, 1 heuristic, 2 always)
   int opt_halo2 = 1;                 // "halo2": halo-patch pair kernel for the mid layers
   int opt_tail_n = 1;                // "tail_n": taps-in-N image-gradient tail
-  int opt_c64_slots = 0;             // "c64_slots": halo ring depth override
-  int opt_halo2_stages = 0;          // "halo2_stages": weight ring depth override
   int opt_smem_reserve_kb = 0;       // "smem_reserve_kb": shared memory the persistent conv CTAs leave free per SM
   int opt_sweep64 = 1;               // "sweep64": tap-stacked sweep kernel for the 64 -> 64 layers (0 never, 1 = default: launches
                                      // whose 128-pixel strips fit the image and give every SM work, 2 always)
-  int opt_sweep_dbg = 0;             // "sweep_dbg": diagnostics of the sweep kernel (wrong results), see conv_sweep.cu
-  int opt_head_ctas = 5;             // "head_ctas": resident CTAs per SM the conv1_1 head is compiled for (5 or 8)
-  int opt_pool_idx = 1;              // "pool_idx": the NST driver routes the max-pool backward through index bytes (0: re-reads
-                                     // the pre-pool activations, which the forward then always stores)
-  int opt_lm_planes = 0;             // "lm_planes": experiment knob of the landmark bit-plane kernel: requests in flight per warp
-                                     // (5, 10, 20; 0 = default 10) + 100 x grid size in halves of a resident wave (0 = default 4)
   unsigned long long launches = 0;   // kernels launched through this context
   IsxProfiler* prof = nullptr;
 };

@@ -435,15 +435,13 @@ extern "C" int isx_eye_landmarks(const void* seg, int seg_dtype, int B, int H, i
   uint32_t* points = reinterpret_cast<uint32_t*>(ws + L.points);
   lm_init_kernel<<<(B + 127) / 128, 128, 0, s>>>(sclera, B);
   ISX_LAUNCH_CHECK();
-  // blocks per frame: TWO resident waves over the batch (measured with the "lm_planes" knob, 128 maps: half a wave 3.4 TB/s,
-  // one 4.1, one and a half 4.1, two 4.4; 5 / 10 / 20 requests in flight per warp make no difference), at least one block, at
-  // most one warp per row
-  const int knob = isx_ctx()->opt_lm_planes;
-  const int u_sel = knob % 100, halves = knob / 100 > 0 ? knob / 100 : 4;
+  // blocks per frame: TWO resident waves over the batch (measured on a B200, 128 maps: half a wave 3.4 TB/s, one 4.1, one and a
+  // half 4.1, two 4.4), at least one block, at most one warp per row.  10 requests in flight per warp (5 / 10 / 20 measured:
+  // no difference).
   auto launch = [&](auto kernel, const auto* segp) -> int {
     int per_sm = 1;
     ISX_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kLmThreads, 0));
-    const int cap_blocks = std::max(1, isx_num_sms() * std::max(1, per_sm) * halves / 2);
+    const int cap_blocks = std::max(1, isx_num_sms() * std::max(1, per_sm) * 2);
     const int bx = std::max(1, std::min(cap_blocks / B, (H + kLmThreads / 32 - 1) / (kLmThreads / 32)));
     const double label_bytes = seg_dtype == 0 ? 8.0 : seg_dtype == 1 ? 1.0 : 4.0;
     isx_prof_begin(ISX_PROF_PLANES, static_cast<double>(B) * H * (W * label_bytes + 2.0 * L.Wu * 4), s);   // labels in, two bit planes out
@@ -454,10 +452,7 @@ extern "C" int isx_eye_landmarks(const void* seg, int seg_dtype, int B, int H, i
   };
   int rc = 0;
   if (seg_dtype == 0) {
-    const long long* p = static_cast<const long long*>(seg);
-    if (u_sel == 5) rc = launch(lm_planes_kernel<long long, 5>, p);
-    else if (u_sel == 20) rc = launch(lm_planes_kernel<long long, 20>, p);
-    else rc = launch(lm_planes_kernel<long long, 10>, p);
+    rc = launch(lm_planes_kernel<long long, 10>, static_cast<const long long*>(seg));
   } else if (seg_dtype == 1) {
     rc = launch(lm_planes_kernel<uint8_t, 10>, static_cast<const uint8_t*>(seg));
   } else {

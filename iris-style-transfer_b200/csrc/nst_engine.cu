@@ -157,10 +157,8 @@ int run_conv_fwd(const isx_nst_config* c, const isx_nst_buffers* b, const Layout
   if (want_pool) {  // MaxPool2d(2,2) of this layer's output rides the conv epilogue
     ISX_REQUIRE(L.H[lv] >= 2 && L.W[lv] >= 2, "nst: cannot pool a %dx%d map", L.H[lv], L.W[lv]);
     a.pool_out = at(b, L.pool[lv]);
-    if (isx_ctx()->opt_pool_idx) {
-      a.pool_idx = atb(b, L.pidx[lv]);
-      a.skip_out = lean && !conv_tapped(c, i);
-    }
+    a.pool_idx = atb(b, L.pidx[lv]);
+    a.skip_out = lean && !conv_tapped(c, i);
   }
   return conv_tc(a, s);
 }
@@ -248,11 +246,10 @@ int run_backward(const isx_nst_config* c, const isx_nst_buffers* b, const Layout
     a.mask_act = mask ? at(b, tap_off(L, id)) : nullptr;
     return conv_tc(a, s);
   };
-  // max-pool + ReLU backward of the pool after conv `conv` (level lv): through the routing bytes the forward left, or
-  // (option "pool_idx" = 0) by re-reading the pre-pool activation
+  // max-pool + ReLU backward of the pool after conv `conv` (level lv), through the routing bytes the forward left: the
+  // pre-pool activation is not read (a lean forward never stores it)
   auto pool_bwd = [&](const bf16* dy, int lv, int conv, bf16* dx) -> int {
-    if (isx_ctx()->opt_pool_idx) return maxpool_bwd_idx(dy, atb(b, L.pidx[lv]), dx, B, L.H[lv], L.W[lv], kCout[conv], s);
-    return maxpool_bwd(dy, at(b, L.act[conv]), dx, B, L.H[lv], L.W[lv], kCout[conv], s);
+    return maxpool_bwd_idx(dy, atb(b, L.pidx[lv]), dx, B, L.H[lv], L.W[lv], kCout[conv], s);
   };
   // gradient w.r.t. a POOL output: out = g (may be NULL) + every source of that pool tap; no ReLU mask (the max-pool
   // backward that follows applies the ReLU mask of the pre-pool activation)

@@ -23,6 +23,21 @@ def test_library_exports_every_declared_symbol():
     assert isinstance(lib.isx_last_error(), bytes)
 
 
+def test_kernel_selection_options():
+    """isx_set_option / isx_get_option know exactly the five kernel-selection options; the names of removed experiment
+    options are refused like any unknown name."""
+    lib = _lib.load()
+    defaults = {b"c64": 1, b"halo2": 1, b"tail_n": 1, b"sweep64": 1, b"smem_reserve_kb": 0}
+    for name, default in defaults.items():
+        v = ctypes.c_int(-1)
+        assert lib.isx_get_option(name, ctypes.byref(v)) == 0 and v.value == default, name
+        assert lib.isx_set_option(name, default) == 0, name
+    for name in (b"pool_idx", b"head_ctas", b"lm_planes", b"sweep_dbg", b"c64_slots", b"halo2_stages"):
+        assert lib.isx_set_option(name, 1) != 0, name
+        assert b"unknown option '%s'" % name in lib.isx_last_error()
+        assert lib.isx_get_option(name, ctypes.byref(ctypes.c_int())) != 0, name
+
+
 def test_header_has_no_torch_types():
     txt = open(_lib.HEADER_PATH).read()
     assert 'extern "C"' in txt
