@@ -365,6 +365,43 @@ int isx_eye_landmarks(const void* seg, int seg_dtype, int B, int H, int W, doubl
 int isx_gaze_head_fwd(const float* x, int64_t ld_x, int B, int in_dim, int hidden, int out_dim, const float* W1, const float* b1,
                       const float* W2, const float* b2, const float* W3, const float* b3, float* out, isx_stream stream);
 
+/* ---- ResNet-50 trunk: the feature extractor of GazeEstimator2(extract_feature=True) (models/gaze_estimators/
+ * gaze_estimators.py:180-223 over models/resnet/resnet.py = torchvision resnet50 without fc, eval mode) -------------------
+ * Activations bf16 NHWC, fp32 accumulation.  BatchNorm is folded into every convolution beforehand (eval mode), so each
+ * layer is conv + bias.  Output sizes round up like torchvision's: a stride-2 layer maps H to ceil(H / 2).
+ * isx_conv_bias_act_fwd: in [B,H,W,Cin] -> out [B,ceil(H/stride),ceil(W/stride),Cout] = relu?(conv(in) + bias [+ residual]);
+ *   k = 1 (pad 0; w from isx_pack_conv1x1_weights) or 3 (pad 1; w_fwd from isx_pack_conv3x3_weights), stride 1 or 2,
+ *   Cin and Cout multiples of 64; residual (may be NULL) has out's shape and is added before the ReLU (Bottleneck.forward).
+ * isx_pack_conv1x1_weights: fp32 [Cout,Cin(,1,1)] -> bf16 [Cout][Cin].
+ * isx_resnet_stem_fwd: conv1 (7x7, stride 2, pad 3, 3 -> 64) + bias + ReLU, straight from the fp32 NCHW image
+ *   x [B,xc,H,W] (xc = 1 broadcasts to three channels) -> bf16 [B,ceil(H/2),ceil(W/2),64]; w from
+ *   isx_pack_resnet_stem_weights (fp32 OIHW [64,3,7,7] -> bf16 [64][192]).
+ * isx_maxpool3x3s2_fwd: MaxPool2d(3, 2, padding 1) bf16 [B,H,W,C] -> [B,ceil(H/2),ceil(W/2),C], C a multiple of 8;
+ *   bit-identical to torch (padding is -inf, the first maximum of the window wins, NaN propagates).
+ * isx_global_avgpool: AdaptiveAvgPool2d(1) + flatten, bf16 [B,HW,C] -> fp32 [B,C]; C a multiple of 8; deterministic. */
+int isx_pack_conv1x1_weights(const float* w, int Cout, int Cin, isx_bf16* w_out, isx_stream stream);
+int isx_pack_resnet_stem_weights(const float* w, isx_bf16* w_out, isx_stream stream);
+int isx_conv_bias_act_fwd(const isx_bf16* in, const isx_bf16* w, const float* bias, const isx_bf16* residual, isx_bf16* out,
+                          int B, int H, int W, int Cin, int Cout, int k, int stride, int relu, isx_stream stream);
+int isx_resnet_stem_fwd(const float* x, int xc, const isx_bf16* w, const float* bias, isx_bf16* out, int B, int H, int W,
+                        isx_stream stream);
+int isx_maxpool3x3s2_fwd(const isx_bf16* in, isx_bf16* out, int B, int H, int W, int C, isx_stream stream);
+int isx_global_avgpool(const isx_bf16* in, float* out, int B, int HW, int C, isx_stream stream);
+/* The whole trunk: x fp32 [B,xc,H,W] (xc in {1,3}, H and W >= 32, no input normalisation) -> feat_out fp32 [B,2048].
+ * weights: the 53 folded (weight, bias) pairs in torchvision module order -- conv1, then per Bottleneck of layer1..layer4
+ * conv1 (1x1), conv2 (3x3, carries the stride), conv3 (1x1), and after the first block's conv3 its downsample.0 (1x1,
+ * strided).  w[0] from isx_pack_resnet_stem_weights, 1x1 from isx_pack_conv1x1_weights, 3x3 the w_fwd of
+ * isx_pack_conv3x3_weights; bias fp32 [Cout].  workspace: isx_resnet50_workspace_bytes(B, H, W) bytes (host-only query;
+ * -1 and isx_last_error for B < 1 or H, W < 32). */
+#define ISX_RESNET50_CONVS 53
+typedef struct {
+  const isx_bf16* w[ISX_RESNET50_CONVS];
+  const float* bias[ISX_RESNET50_CONVS];
+} isx_resnet50_weights;
+int64_t isx_resnet50_workspace_bytes(int B, int H, int W);
+int isx_resnet50_forward(const isx_resnet50_weights* weights, const float* x, int xc, int B, int H, int W, void* workspace,
+                         float* feat_out, isx_stream stream);
+
 /* ---- evaluation metrics of the drivers ------------------------------------------------------------------------------------
  * isx_seg_iou = utils.cal_IoUs (utils.py:163-194; iris_style_transfer_openeds2019.py:156, data_preprocessing.py:168): preds,
  * targets int64 [B,HW] label maps -> iou fp32 [B,num_class] = intersection / (union + eps) per image and class, miou fp32 [B] =

@@ -14,6 +14,7 @@ try:  # torch-dependent surface (the ctypes layer and the synthetic generators i
     from .frames import stylize_frames  # noqa: F401
     from .ritnet import RITnet  # noqa: F401
     from .classifiers import Classifier1, Classifier2  # noqa: F401
+    from .resnet import ResNet50  # noqa: F401
     from .gaze import (GazeEstimator1, GazeEstimator2, extract_eye_landmarks,  # noqa: F401
                        extract_eye_landmarks_batch)
     from . import features, frames, sharding  # noqa: F401

@@ -98,7 +98,7 @@ static EncodeTiledFn get_encode_fn() {
 }
 
 int isx_make_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims,
-                       const uint64_t* strides_bytes, const uint32_t* box, bool swizzle128) {
+                       const uint64_t* strides_bytes, const uint32_t* box, bool swizzle128, const uint32_t* elem_strides) {
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) return 3;
   cuuint64_t gdim[5];
@@ -108,7 +108,7 @@ int isx_make_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint6
   for (int i = 0; i < rank; ++i) {
     gdim[i] = dims[i];
     bx[i] = box[i];
-    es[i] = 1;
+    es[i] = elem_strides ? elem_strides[i] : 1;
   }
   for (int i = 0; i + 1 < rank; ++i) gstr[i] = strides_bytes[i];
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) {

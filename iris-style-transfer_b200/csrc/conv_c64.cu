@@ -461,7 +461,7 @@ static int launch_c64(const ConvArgs& a, cudaStream_t stream) {
 
 // Cin = 64, 3x3, shared weights, Cout 64 (bf16 NHWC out) or the N = 16 image-gradient tail.
 bool conv_c64_applicable(const ConvArgs& a) {
-  if (a.Cin != 64 || a.ntaps != 9 || a.per_image_weights) return false;
+  if (a.Cin != 64 || a.ntaps != 9 || a.per_image_weights || a.stride != 1) return false;
   if (a.dx_nchw != nullptr) return a.Cout == 16;
   if (a.Cout != 64) return false;
   if (a.gram_act != nullptr && a.gram_act != a.mask_act) return false;

@@ -498,7 +498,7 @@ static double pair_efficiency(int H, int W, int pw, int ph) {
 }
 
 bool conv_halo_applicable(const ConvArgs& a) {
-  if (a.ntaps != 9 || a.per_image_weights || a.dx_nchw != nullptr) return false;
+  if (a.ntaps != 9 || a.per_image_weights || a.dx_nchw != nullptr || a.stride != 1) return false;
   if (a.Cin % 64 != 0 || a.Cout % 64 != 0) return false;
   if (a.out == nullptr) return false;
   return true;

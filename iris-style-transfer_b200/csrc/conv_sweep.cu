@@ -640,7 +640,7 @@ conv_sweep64_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 static double strip_efficiency(int n) { return static_cast<double>(n) / (((n + 127) / 128) * 128); }
 
 bool conv_sweep_applicable(const ConvArgs& a) {
-  if (a.Cin != 64 || a.Cout != 64 || a.ntaps != 9 || a.per_image_weights || a.dx_nchw != nullptr) return false;
+  if (a.Cin != 64 || a.Cout != 64 || a.ntaps != 9 || a.per_image_weights || a.dx_nchw != nullptr || a.stride != 1) return false;
   if (a.out == nullptr) return false;
   if (a.gram_act != nullptr && a.gram_act != a.mask_act) return false;
   if (a.aff_a != nullptr && a.mask_act == nullptr) return false;

@@ -1,4 +1,4 @@
-// K1 / K3 / K5: 3x3 (stride 1, pad 1) and 1x1 convolutions over NHWC bf16 activations as an
+// K1 / K3 / K5: 3x3 (pad 1) and 1x1 convolutions, stride 1 or 2, over NHWC bf16 activations as an
 // implicit GEMM on the 5th-gen tensor cores (tcgen05.mma, fp32 accumulators in TMEM), operands
 // staged by TMA.  One kernel covers
 //   * conv fwd + bias + ReLU                      (reference: torchvision vgg19.features Conv2d+ReLU,
@@ -11,6 +11,9 @@
 // N = Cout tile (BN), K = ntaps * Cin walked as (tap, 64-channel chunk).  For every K block the
 // producer issues one 4-D TMA box load per M-tile at the tap-shifted coordinate (out-of-bounds
 // rows/cols are zero-filled by TMA == the conv's zero padding) and one 2-D load of the weight slab.
+// Stride 2 (ResNet-50 bottlenecks, torchvision resnet50 via models/gaze_estimators/gaze_estimators.py:180-223): the
+// activation map traverses W and H with element stride 2, so a 2TW x 2TH box starting at (2 x0 + kx - 1, 2 y0 + ky - 1)
+// lands the TW x TH input pixels of the output patch in the same swizzled tile.
 // The A/B tiles land in the SWIZZLE_128B K-major layout tcgen05 consumes directly.
 //
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer,
@@ -23,8 +26,9 @@
 namespace isx {
 
 struct ConvParams {
-  int B, H, W, Cin, Cout;
+  int B, H, W, Cin, Cout;    // H, W: OUTPUT size (the input is stride x larger, rounded up)
   int ntaps;                 // 9 or 1
+  int stride;                // 1 or 2
   int TW, TH, TB;            // patch shape, TW*TH*TB == 128
   int tiles_x, tiles_y, tiles_b;
   int n_tiles;               // Cout / BN
@@ -122,6 +126,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // ================================ TMA producer =========================================
     if (lane == 0) {
       const int wrow0 = (p.w_rows_per_image ? b0[0] * p.w_rows_per_image : 0) + n0;
+      const int stride = EPI == 0 ? p.stride : 1;  // the image-gradient tail is stride 1
       // running stage / tap / channel-block counters (no division on the producer's critical path)
       int s = 0, tap = 0, cb = 0, ky = p.ntaps == 9 ? 0 : 1, kx = p.ntaps == 9 ? 0 : 1;
       uint32_t ph = 0;
@@ -134,7 +139,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (kb < num_kb_conv) {
 #pragma unroll
           for (int mt = 0; mt < MT; ++mt)
-            tma_load_4d(st + mt * kATileBytes, &tmA, &full_bar[sb], cb * 64, x0[mt] + kx - 1, y0[mt] + ky - 1, b0[mt]);
+            tma_load_4d(st + mt * kATileBytes, &tmA, &full_bar[sb], cb * 64, x0[mt] * stride + kx - 1,
+                        y0[mt] * stride + ky - 1, b0[mt]);
           tma_load_2d(st + MT * kATileBytes, &tmB, &full_bar[sb], cb * 64, tap * p.Cout + wrow0);
           if (++cb == cin_blocks) {
             cb = 0; ++tap;
@@ -384,11 +390,12 @@ template <int BN, int MT, int EPI = 0>
 static int launch_conv(const ConvArgs& a, int stages_override, cudaStream_t stream) {
   ConvParams p;
   memset(&p, 0, sizeof(p));
-  p.B = a.B; p.H = a.H; p.W = a.W; p.Cin = a.Cin; p.Cout = a.Cout; p.ntaps = a.ntaps;
+  const int Ho = (a.H + a.stride - 1) / a.stride, Wo = (a.W + a.stride - 1) / a.stride;  // output size
+  p.B = a.B; p.H = Ho; p.W = Wo; p.Cin = a.Cin; p.Cout = a.Cout; p.ntaps = a.ntaps; p.stride = a.stride;
   const bool per_image = a.per_image_weights || a.gram_act != nullptr;
-  choose_patch(a.B, a.H, a.W, per_image, &p.TW, &p.TH, &p.TB);
-  p.tiles_x = (a.W + p.TW - 1) / p.TW;
-  p.tiles_y = (a.H + p.TH - 1) / p.TH;
+  choose_patch(a.B, Ho, Wo, per_image, &p.TW, &p.TH, &p.TB);
+  p.tiles_x = (Wo + p.TW - 1) / p.TW;
+  p.tiles_y = (Ho + p.TH - 1) / p.TH;
   p.tiles_b = (a.B + p.TB - 1) / p.TB;
   p.n_tiles = a.Cout / BN;
   p.w_rows_per_image = a.per_image_weights ? a.Cout : 0;
@@ -422,8 +429,9 @@ static int launch_conv(const ConvArgs& a, int stages_override, cudaStream_t stre
   {
     uint64_t dims[4] = {(uint64_t)a.Cin, (uint64_t)a.W, (uint64_t)a.H, (uint64_t)a.B};
     uint64_t str[3] = {(uint64_t)a.Cin * 2, (uint64_t)a.W * a.Cin * 2, (uint64_t)a.H * a.W * a.Cin * 2};
-    uint32_t box[4] = {64, (uint32_t)p.TW, (uint32_t)p.TH, (uint32_t)p.TB};
-    if (isx_make_tmap_bf16(&tmA, a.in, 4, dims, str, box, true)) return 3;
+    uint32_t box[4] = {64, (uint32_t)(p.TW * a.stride), (uint32_t)(p.TH * a.stride), (uint32_t)p.TB};
+    const uint32_t es[4] = {1, (uint32_t)a.stride, (uint32_t)a.stride, 1};
+    if (isx_make_tmap_bf16(&tmA, a.in, 4, dims, str, box, true, es)) return 3;
   }
   {
     uint64_t rows = (uint64_t)a.ntaps * a.Cout * (a.per_image_weights ? a.B : 1);
@@ -433,8 +441,8 @@ static int launch_conv(const ConvArgs& a, int stages_override, cudaStream_t stre
     if (isx_make_tmap_bf16(&tmB, a.weight, 2, dims, str, box, true)) return 3;
   }
   if (EPI == 0) {
-    uint64_t dims[4] = {(uint64_t)a.Cout, (uint64_t)a.W, (uint64_t)a.H, (uint64_t)a.B};
-    uint64_t str[3] = {(uint64_t)a.Cout * 2, (uint64_t)a.W * a.Cout * 2, (uint64_t)a.H * a.W * a.Cout * 2};
+    uint64_t dims[4] = {(uint64_t)a.Cout, (uint64_t)Wo, (uint64_t)Ho, (uint64_t)a.B};
+    uint64_t str[3] = {(uint64_t)a.Cout * 2, (uint64_t)Wo * a.Cout * 2, (uint64_t)Ho * Wo * a.Cout * 2};
     uint32_t box[4] = {64, (uint32_t)p.TW, (uint32_t)p.TH, (uint32_t)p.TB};
     if (isx_make_tmap_bf16(&tmO, a.out, 4, dims, str, box, true)) return 3;
   } else {
@@ -468,7 +476,7 @@ static int launch_conv(const ConvArgs& a, int stages_override, cudaStream_t stre
   auto kern = conv_tc_kernel<BN, MT, EPI>;
   ISX_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
   isx_prof_begin(ISX_PROF_CONV,
-                 2.0 * (a.ntaps * a.Cin + (a.gram_act ? a.Cout : 0)) * a.Cout * static_cast<double>(a.B) * a.H * a.W, stream);
+                 2.0 * (a.ntaps * a.Cin + (a.gram_act ? a.Cout : 0)) * a.Cout * static_cast<double>(a.B) * Ho * Wo, stream);
   kern<<<(unsigned)grid, kConvThreads, smem_bytes, stream>>>(tmA, tmB, tmO, tmM, tmA2, tmB2, tmP, p);
   isx_prof_end(ISX_PROF_CONV, stream);
   ISX_LAUNCH_CHECK();
@@ -481,10 +489,14 @@ static int launch_conv(const ConvArgs& a, int stages_override, cudaStream_t stre
 
 int conv_tc(const ConvArgs& a_in, cudaStream_t stream) {
   ConvArgs a = a_in;
+  ISX_REQUIRE(a.stride == 1 || (a.stride == 2 && a.pool_out == nullptr && a.mask_act == nullptr && a.gram_act == nullptr &&
+                                a.dx_nchw == nullptr && !a.per_image_weights),
+              "conv_tc: stride %d (stride 2 is the plain forward conv: no pool, mask, image gradient or per-image weights)",
+              a.stride);
   if (a.dx_nchw != nullptr && isx_ctx()->opt_tail_n > 0 && isx_ctx()->opt_c64 < 2 && a.force_bn == 0 &&
       a.Cin == 64 && a.Cout == 16 && a.ntaps == 9)
     return conv1_1_tail_n(a.in, a.weight, a.in_mask, a.mask_b, a.dx_nchw, a.xc, a.B, a.H, a.W, stream);
-  if (isx_ctx()->opt_sweep64 > 0 && a.force_bn == 0 && conv_sweep_applicable(a)) {
+  if (isx_ctx()->opt_sweep64 > 0 && a.force_bn == 0 && !a.generic_only && conv_sweep_applicable(a)) {
     // strips of 128 pixels along the better-fitting image axis, every CTA sweeps an equal share of them: worth it when the
     // strips are mostly real pixels (the kernel is ~1.5x faster per processed pixel than conv_c64) and every SM gets a few
     // hundred of them (a CTA's share starts and ends with two slower edge strips)
@@ -496,10 +508,10 @@ int conv_tc(const ConvArgs& a_in, cudaStream_t stream) {
         (conv_sweep_efficiency(a) >= 0.85 && strips >= 64L * kNumSMs && std::min(a.H, a.W) >= 16))
       return conv_sweep(a, stream);
   }
-  if (isx_ctx()->opt_c64 > 0 && a.force_bn == 0 && conv_c64_applicable(a) &&
+  if (isx_ctx()->opt_c64 > 0 && a.force_bn == 0 && !a.generic_only && conv_c64_applicable(a) &&
       (isx_ctx()->opt_c64 >= 2 || (a.dx_nchw == nullptr && static_cast<long>(a.B) * ((a.H + 15) / 16) * ((a.W + 7) / 8) >= kNumSMs)))
     return conv_c64(a, stream);
-  if (isx_ctx()->opt_halo2 > 0 && a.force_bn == 0 && conv_halo_applicable(a)) {
+  if (isx_ctx()->opt_halo2 > 0 && a.force_bn == 0 && !a.generic_only && conv_halo_applicable(a)) {
     const long items = static_cast<long>(a.B) * ((a.H + 15) / 16) * ((a.W + 15) / 16) * (a.Cout / (a.Cout % 128 == 0 ? 128 : 64));
     if (isx_ctx()->opt_halo2 >= 2 || (items >= 2 * kNumSMs && conv_halo_efficiency(a) >= 0.85)) return conv_halo(a, stream);
   }
@@ -527,7 +539,7 @@ int conv_tc(const ConvArgs& a_in, cudaStream_t stream) {
     mt = (bn == 256 || a.per_image_weights) ? 1 : 2;
     if (st == 0) st = 2;
     // small problems: prefer more CTAs over bigger tiles
-    const long pix_tiles = (static_cast<long>(a.B) * a.H * a.W + 127) / 128;
+    const long pix_tiles = (static_cast<long>(a.B) * ((a.H + a.stride - 1) / a.stride) * ((a.W + a.stride - 1) / a.stride) + 127) / 128;
     auto ctas = [&](int BN_, int MT_) { return ((pix_tiles + MT_ - 1) / MT_) * (a.Cout / BN_); };
     if (ctas(bn, mt) < 2 * kNumSMs && mt == 2) mt = 1;
     if (ctas(bn, mt) < 2 * kNumSMs && bn == 256) bn = 128;

@@ -66,8 +66,11 @@ enum { ISX_PROF_CONV = 0, ISX_PROF_GRAM = 1, ISX_PROF_LBFGS = 2, ISX_PROF_PLANES
 
 // Encode a tiled bf16 tensor map (rank <= 5).  dims/strides innermost first; strides in BYTES
 // for dims 1..rank-1 (dim 0 is contiguous).  swizzle128: CU_TENSOR_MAP_SWIZZLE_128B else NONE.
+// elem_strides (NULL = all 1): traversal stride per dim -- a box then lands ceil(box[i] / elem_strides[i]) elements of
+// dim i, those at start, start + s, start + 2s, ... (strided convolutions).
 int isx_make_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims,
-                       const uint64_t* strides_bytes, const uint32_t* box, bool swizzle128);
+                       const uint64_t* strides_bytes, const uint32_t* box, bool swizzle128,
+                       const uint32_t* elem_strides = nullptr);
 
 #ifdef __CUDACC__
 namespace isx {

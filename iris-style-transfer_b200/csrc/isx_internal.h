@@ -12,6 +12,9 @@ struct ConvArgs {
   const __nv_bfloat16* weight = nullptr;  // [ntaps][Cout][Cin] (x B when per_image_weights)
   __nv_bfloat16* out = nullptr;           // [B,H,W,Cout]
   int B = 0, H = 0, W = 0, Cin = 0, Cout = 0, ntaps = 9;
+  // 1 or 2 (generic kernel only): out is [B, ceil(H/stride), ceil(W/stride), Cout], pixel (x, y) reads input
+  // (stride*x + kx - 1, stride*y + ky - 1) for the 3x3 taps and (stride*x, stride*y) for ntaps = 1
+  int stride = 1;
   bool per_image_weights = false;
   const float* bias = nullptr;
   int relu = 0;
@@ -26,6 +29,9 @@ struct ConvArgs {
   const float* aff_a = nullptr;
   const float* aff_b = nullptr;
   int force_bn = 0, force_mt = 0, force_stages = 0;  // tuning / test hooks (0 = heuristic)
+  // generic kernel only: the specialised 3x3 kernels sum in another order and are picked by the batch size, so a caller
+  // whose results must not depend on the batch (ResNet-50 features: image i of a batch == image i alone) skips them
+  bool generic_only = false;
   // fused Gram backward: out += gram_act . gram_D[b]   (gram_act [B,H,W,Cout], gram_D bf16 [B,Cout,Cout])
   const __nv_bfloat16* gram_act = nullptr;
   const __nv_bfloat16* gram_D = nullptr;

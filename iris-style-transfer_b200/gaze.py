@@ -3,8 +3,9 @@ device for whole batches of label maps, and the GazeEstimator1 / GazeEstimator2 
 
 The reference extracts the 19 landmarks one frame at a time with a `.cpu().numpy()` round trip and three OpenCV calls per
 class (gaze_estimators.py:49,127-137); here a batch is three kernel launches and never leaves the device.  Training the
-heads (gaze_estimation.py, Adam) and the ResNet50 / EfficientNet feature extractors stay with the caller (out of the
-accelerated path, SURVEY.md §2): `GazeEstimator2(extract_feature=True)` needs a `resnet=` callable."""
+heads (gaze_estimation.py, Adam) and the EfficientNet segmenter stay with the caller (SURVEY.md §2).
+`GazeEstimator2(extract_feature=True)` takes its feature extractor as `resnet=`: `iris_b200.ResNet50` keeps frames ->
+features -> head -> unit vectors on the device."""
 from __future__ import annotations
 
 from typing import Callable, Dict, Optional
@@ -113,16 +114,17 @@ class GazeEstimator1(_GazeHead):
 
 
 class GazeEstimator2(_GazeHead):
-    """gaze_estimators.py:180-223: the appearance-based estimator on 2048 ResNet50 features.  The feature extractor itself
-    (models/resnet/resnet.py, ImageNet weights) is outside the accelerated path: pass it as `resnet=` when extract_feature."""
+    """gaze_estimators.py:180-223: the appearance-based estimator on 2048 ResNet50 features.  With extract_feature the
+    feature extractor (models/resnet/resnet.py) is passed as `resnet=`, e.g. `iris_b200.ResNet50(weights=<torchvision
+    resnet50 module or state dict>)`; it applies no input normalisation, so frames arrive preprocessed."""
 
     def __init__(self, extract_feature: bool = False, freeze_resnet: bool = True, hidden_dim: int = 64, output_dim: int = 3,
                  state_dict: Optional[Dict[str, torch.Tensor]] = None, resnet: Optional[Callable] = None):
         super().__init__(2048, hidden_dim, output_dim, state_dict)
         self.extract_feature = extract_feature
         if extract_feature and resnet is None:
-            raise ValueError("GazeEstimator2(extract_feature=True) needs resnet=<callable image -> [B,2048] features>: ResNet50 "
-                             "is not part of this library (SURVEY.md §2, out of scope)")
+            raise ValueError("GazeEstimator2(extract_feature=True) needs resnet=<callable image -> [B,2048] features>, e.g. "
+                             "iris_b200.ResNet50(weights=<torchvision resnet50 module or state dict>)")
         self._resnet = resnet
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
