@@ -295,6 +295,11 @@ int isx_nst_eval(const isx_nst_config* cfg, const isx_nst_buffers* bufs, const f
  * raises on the empty min()).  Bit-exact integer work. */
 int isx_mask_bbox(const float* x, const int64_t* seg, int label, int use_threshold, float threshold, uint8_t* mask,
                   float* xm, int32_t* bbox, int B, int H, int W, isx_stream stream);
+/* isx_mask_bbox for a label map of either dtype: seg_dtype 0 = int64 (= isx_mask_bbox), 1 = uint8 [B,1,H,W], compared as
+ * int(seg) == label, so the result equals the int64 call on the widened map (a label outside 0..255 matches nothing).  Any
+ * other seg_dtype is an error. */
+int isx_mask_bbox_typed(const float* x, const void* seg, int seg_dtype, int label, int use_threshold, float threshold,
+                        uint8_t* mask, float* xm, int32_t* bbox, int B, int H, int W, isx_stream stream);
 /* torchvision v2 Resize (bilinear, antialias=True) of the window src_bbox (or the whole image when NULL) of
  * src fp32 [B,src_c,SH,SW] to dst fp32 [B,dst_c,DH,DW]; src_c == 3 is converted to gray first
  * (rgb_to_grayscale, …2019.py:112); the single result channel is replicated dst_c times (…2019.py:79). */
@@ -328,6 +333,11 @@ int64_t isx_ritnet_param_floats(void);
 int64_t isx_ritnet_workspace_bytes(int B, int H, int W);
 int isx_ritnet_forward(const float* x, const float* params, const uint8_t* gamma_lut, const float* norm_lut, void* workspace,
                        int64_t* labels, float* logits, int B, int H, int W, isx_stream stream);
+/* isx_ritnet_forward writing labels of label_dtype 0 = int64 (= isx_ritnet_forward) or 1 = uint8 [B,H,W] (same values, 1 B
+ * per pixel); any other label_dtype is an error.  The logits do not depend on it. */
+int isx_ritnet_forward_typed(const float* x, const float* params, const uint8_t* gamma_lut, const float* norm_lut,
+                             void* workspace, void* labels, int label_dtype, float* logits, int B, int H, int W,
+                             isx_stream stream);
 
 /* ---- classifier heads (models/classifiers/classifiers.py:3-72; iris_classification.py:66-71, …2019.py:82-84) -----------
  * A Linear layer over a batch of M <= 256 eyes is a weight-streaming tcgen05 GEMM out^T[N,M] = W'[N,K'] . X'[M,K']^T with
@@ -410,6 +420,11 @@ int isx_resnet50_forward(const isx_resnet50_weights* weights, const float* x, in
  * isx_angular_distance = utils.angular_distance (utils.py:216-240): rows v1, v2 fp32 [n,d] -> acos(clamp(<v1,v2>)) and degrees. */
 int isx_seg_iou(const int64_t* preds, const int64_t* targets, int B, int64_t HW, int num_class, float eps, uint32_t* counts,
                 float* iou, float* miou, isx_stream stream);
+/* isx_seg_iou for two label maps of the same dtype: seg_dtype 0 = int64 (= isx_seg_iou), 1 = uint8 [B,HW] (2 B per pixel
+ * instead of 16; any alignment and HW).  The counts are exact either way, so the results are bit-identical to the int64 call
+ * on the widened maps.  Any other seg_dtype is an error. */
+int isx_seg_iou_typed(const void* preds, const void* targets, int seg_dtype, int B, int64_t HW, int num_class, float eps,
+                      uint32_t* counts, float* iou, float* miou, isx_stream stream);
 int isx_angular_distance(const float* v1, const float* v2, int n, int d, float* radian, float* degree, isx_stream stream);
 
 /* ---- measurement hooks (bench.py) -------------------------------------------------------------

@@ -9,6 +9,7 @@
 // pixels the mask discards.
 #include <algorithm>
 #include <limits.h>
+#include <type_traits>
 
 #include "../../include/isx.h"
 #include "isx_common.cuh"
@@ -24,12 +25,15 @@ __global__ void bbox_init_kernel(int32_t* bbox, int B) {
 }
 
 // m = (seg == label) & (x <= thr)   [either test may be disabled]; xm = x * m; bbox over xm != 0.
-// VEC = 4: four pixels per thread (float4 / 2 x longlong2 loads, uchar4 / float4 stores); needs W % 4 == 0 and
-// 16-byte aligned rows, which the launcher checks.
-template <int VEC>
+// T = int64_t or uint8_t label maps; a uint8 label compares as int(seg) == label, so the result equals the int64 path on the
+// widened map for every label (one outside 0..255 matches nothing).
+// VEC = 4: four pixels per thread (float4 loads, 2 x longlong2 or one uchar4 label load, uchar4 / float4 stores); needs
+// W % 4 == 0, 16-byte aligned x / xm and int64 rows, 4-byte aligned uint8 rows, which the launcher checks.
+template <int VEC, typename T>
 __global__ void __launch_bounds__(256)
-mask_bbox_kernel(const float* __restrict__ x, const int64_t* __restrict__ seg, int label, int use_thr, float thr,
+mask_bbox_kernel(const float* __restrict__ x, const T* __restrict__ seg, int label, int use_thr, float thr,
                  uint8_t* __restrict__ mask, float* __restrict__ xm, int32_t* __restrict__ bbox, int H, int W) {
+  using Lab = typename std::conditional<sizeof(T) == 8, long long, int>::type;
   const int b = blockIdx.y;
   const long hw = static_cast<long>(H) * W;
   const long nv = hw / VEC;
@@ -38,14 +42,19 @@ mask_bbox_kernel(const float* __restrict__ x, const int64_t* __restrict__ seg, i
        i += static_cast<long>(gridDim.x) * blockDim.x) {
     const long e = i * VEC;
     float v[VEC];
-    long long sg[VEC];
+    Lab sg[VEC];
     if (VEC == 4) {
       const float4 q = __ldg(reinterpret_cast<const float4*>(x + b * hw + e));
       v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
       if (seg) {
-        const longlong2 s0 = __ldg(reinterpret_cast<const longlong2*>(seg + b * hw + e));
-        const longlong2 s1 = __ldg(reinterpret_cast<const longlong2*>(seg + b * hw + e + 2));
-        sg[0] = s0.x; sg[1] = s0.y; sg[2] = s1.x; sg[3] = s1.y;
+        if constexpr (sizeof(T) == 8) {
+          const longlong2 s0 = __ldg(reinterpret_cast<const longlong2*>(seg + b * hw + e));
+          const longlong2 s1 = __ldg(reinterpret_cast<const longlong2*>(seg + b * hw + e + 2));
+          sg[0] = s0.x; sg[1] = s0.y; sg[2] = s1.x; sg[3] = s1.y;
+        } else {
+          const uchar4 s0 = __ldg(reinterpret_cast<const uchar4*>(seg + b * hw + e));
+          sg[0] = s0.x; sg[1] = s0.y; sg[2] = s0.z; sg[3] = s0.w;
+        }
       }
     } else {
       v[0] = x[b * hw + e];
@@ -210,24 +219,38 @@ static int launch_resize(const float* src, int src_c, int SH, int SW, const int3
 using namespace isx;
 static inline cudaStream_t S(isx_stream s) { return reinterpret_cast<cudaStream_t>(s); }
 
-extern "C" int isx_mask_bbox(const float* x, const int64_t* seg, int label, int use_threshold, float threshold,
-                             uint8_t* mask, float* xm, int32_t* bbox, int B, int H, int W, isx_stream stream) {
+extern "C" int isx_mask_bbox_typed(const float* x, const void* seg, int seg_dtype, int label, int use_threshold, float threshold,
+                                   uint8_t* mask, float* xm, int32_t* bbox, int B, int H, int W, isx_stream stream) {
+  ISX_REQUIRE(seg_dtype == 0 || seg_dtype == 1, "isx_mask_bbox: seg_dtype %d (0 = int64, 1 = uint8)", seg_dtype);
   ISX_REQUIRE(x && bbox && B > 0 && H > 0 && W > 0, "isx_mask_bbox: bad arguments");
   bbox_init_kernel<<<(B + 127) / 128, 128, 0, S(stream)>>>(bbox, B);
   ISX_LAUNCH_CHECK();
   const long hw = static_cast<long>(H) * W;
   auto al16 = [](const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
-  const bool vec = (W % 4 == 0) && al16(x) && al16(seg) && al16(xm) && (mask == nullptr || (reinterpret_cast<uintptr_t>(mask) & 3) == 0);
+  const bool u8 = seg_dtype == 1;
+  const bool seg_al = u8 ? (reinterpret_cast<uintptr_t>(seg) & 3) == 0 : al16(seg);
+  const bool vec = (W % 4 == 0) && al16(x) && seg_al && al16(xm) && (mask == nullptr || (reinterpret_cast<uintptr_t>(mask) & 3) == 0);
   const long items = vec ? hw / 4 : hw;
   // whole waves of 256-thread blocks: 148 SMs x 8 resident blocks, split over the images
   const int bx = static_cast<int>(std::min<long>((items + 255) / 256, std::max<long>(1, static_cast<long>(isx_num_sms()) * 8 / B)));
   dim3 grid(bx, B);
-  if (vec)
-    mask_bbox_kernel<4><<<grid, 256, 0, S(stream)>>>(x, seg, label, use_threshold, threshold, mask, xm, bbox, H, W);
+  const int64_t* s64 = static_cast<const int64_t*>(seg);
+  const uint8_t* s8 = static_cast<const uint8_t*>(seg);
+  if (u8 && vec)
+    mask_bbox_kernel<4, uint8_t><<<grid, 256, 0, S(stream)>>>(x, s8, label, use_threshold, threshold, mask, xm, bbox, H, W);
+  else if (u8)
+    mask_bbox_kernel<1, uint8_t><<<grid, 256, 0, S(stream)>>>(x, s8, label, use_threshold, threshold, mask, xm, bbox, H, W);
+  else if (vec)
+    mask_bbox_kernel<4, int64_t><<<grid, 256, 0, S(stream)>>>(x, s64, label, use_threshold, threshold, mask, xm, bbox, H, W);
   else
-    mask_bbox_kernel<1><<<grid, 256, 0, S(stream)>>>(x, seg, label, use_threshold, threshold, mask, xm, bbox, H, W);
+    mask_bbox_kernel<1, int64_t><<<grid, 256, 0, S(stream)>>>(x, s64, label, use_threshold, threshold, mask, xm, bbox, H, W);
   ISX_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int isx_mask_bbox(const float* x, const int64_t* seg, int label, int use_threshold, float threshold,
+                             uint8_t* mask, float* xm, int32_t* bbox, int B, int H, int W, isx_stream stream) {
+  return isx_mask_bbox_typed(x, seg, 0, label, use_threshold, threshold, mask, xm, bbox, B, H, W, stream);
 }
 
 extern "C" int isx_resize_bilinear_aa(const float* src, int src_c, int SH, int SW, const int32_t* src_bbox, float* dst,

@@ -230,9 +230,11 @@ __global__ void rit_avgpool_kernel(const float* __restrict__ in, float* __restri
   }
 }
 
-// out_conv1 (1x1, 32 -> 4, ritnet.py:195) fused with `_, x = x.max(1)` (ritnet.py:55): first maximal class wins
+// out_conv1 (1x1, 32 -> 4, ritnet.py:195) fused with `_, x = x.max(1)` (ritnet.py:55): first maximal class wins.
+// T = int64_t (the reference's dtype) or uint8_t (1 B per pixel for the consumers that read uint8 maps natively).
+template <typename T>
 __global__ void rit_classify_kernel(const float* __restrict__ x9, const float* __restrict__ w, const float* __restrict__ bias,
-                                    int64_t* __restrict__ labels, float* __restrict__ logits, long hw, long npix) {
+                                    T* __restrict__ labels, float* __restrict__ logits, long hw, long npix) {
   for (long i = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x; i < npix; i += static_cast<long>(gridDim.x) * blockDim.x) {
     float l[4] = {__ldg(bias), __ldg(bias + 1), __ldg(bias + 2), __ldg(bias + 3)};
     const float4* s = reinterpret_cast<const float4*>(x9 + i * 32);
@@ -248,7 +250,7 @@ __global__ void rit_classify_kernel(const float* __restrict__ x9, const float* _
     int best = 0;
 #pragma unroll
     for (int k = 1; k < 4; ++k) if (l[k] > l[best]) best = k;
-    labels[i] = best;
+    labels[i] = static_cast<T>(best);
     if (logits) {
       const long b = i / hw, p = i - b * hw;
 #pragma unroll
@@ -358,8 +360,10 @@ extern "C" int isx_ritnet_transform(const float* x, const uint8_t* gamma_lut, co
                        reinterpret_cast<uint8_t*>(ws + rit_align(static_cast<size_t>(B) * H * W)), out, B, H, W, S(stream));
 }
 
-extern "C" int isx_ritnet_forward(const float* x, const float* params, const uint8_t* gamma_lut, const float* norm_lut,
-                                  void* workspace, int64_t* labels, float* logits, int B, int H, int W, isx_stream stream) {
+extern "C" int isx_ritnet_forward_typed(const float* x, const float* params, const uint8_t* gamma_lut, const float* norm_lut,
+                                        void* workspace, void* labels, int label_dtype, float* logits, int B, int H, int W,
+                                        isx_stream stream) {
+  ISX_REQUIRE(label_dtype == 0 || label_dtype == 1, "isx_ritnet_forward: label_dtype %d (0 = int64, 1 = uint8)", label_dtype);
   ISX_REQUIRE(x && params && gamma_lut && norm_lut && workspace && labels, "isx_ritnet_forward: null pointer");
   ISX_REQUIRE(B > 0 && H >= 16 && W >= 16 && H % 16 == 0 && W % 16 == 0,
               "isx_ritnet_forward: frame %dx%d must be a positive multiple of 16 in both dimensions (four 2x2 poolings and "
@@ -410,8 +414,18 @@ extern "C" int isx_ritnet_forward(const float* x, const float* params, const uin
     if (int rc = launch_conv(P.up[k][3], params, t, none, none, 1, 1, nullptr, nullptr, buf[l][3], B, h, w, s)) return rc;      // out
     prev = buf[l][3];
   }
-  rit_classify_kernel<<<static_cast<int>(std::min<long>((n + 255) / 256, static_cast<long>(isx_num_sms()) * 16)), 256, 0, s>>>(prev, params + P.out_w, params + P.out_b, labels, logits,
-                                                                                                   static_cast<long>(hw), n);
+  const int cblocks = static_cast<int>(std::min<long>((n + 255) / 256, static_cast<long>(isx_num_sms()) * 16));
+  if (label_dtype == 1)
+    rit_classify_kernel<uint8_t><<<cblocks, 256, 0, s>>>(prev, params + P.out_w, params + P.out_b, static_cast<uint8_t*>(labels),
+                                                         logits, static_cast<long>(hw), n);
+  else
+    rit_classify_kernel<int64_t><<<cblocks, 256, 0, s>>>(prev, params + P.out_w, params + P.out_b, static_cast<int64_t*>(labels),
+                                                         logits, static_cast<long>(hw), n);
   ISX_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int isx_ritnet_forward(const float* x, const float* params, const uint8_t* gamma_lut, const float* norm_lut,
+                                  void* workspace, int64_t* labels, float* logits, int B, int H, int W, isx_stream stream) {
+  return isx_ritnet_forward_typed(x, params, gamma_lut, norm_lut, workspace, labels, 0, logits, B, H, W, stream);
 }

@@ -45,8 +45,8 @@ def stylize_frames(frames: torch.Tensor,
                    inplace: bool = False,
                    **nst_kw):
     """frames: [B,1,H,W] fp32 eye frames (host or device); style_iris: what the drivers hand to nst() as the style --
-    (1,h,w) / (3,h,w) unbatched like …2020.py:103-104, or [B|1,1|3,h,w]; segs: int64 label maps [B,1,H,W] (or
-    `segmenter`).  Returns (new_frames [B,1,H,W] on the device, info) with info = {masks, bboxes, valid, irises,
+    (1,h,w) / (3,h,w) unbatched like …2020.py:103-104, or [B|1,1|3,h,w]; segs: label maps [B,1,H,W], host or device
+    (int64 and uint8 are read as they are, uint8 moves 1 B per pixel; or `segmenter`, e.g. iris_b200.RITnet).  Returns (new_frames [B,1,H,W] on the device, info) with info = {masks, bboxes, valid, irises,
     c_loss_hist, s_loss_hist, evals, timings_ms}.  Frames without a single iris pixel are returned unchanged
     (valid[i] False; the reference would fail in crop_image)."""
     dev = torch.device(device)

@@ -531,7 +531,8 @@ def mask_and_crop_iris(x: torch.Tensor,
     """pipelines.py:112-166: m = (ritnet(x) == 2) * (x <= glint_threshold); x*m; trim to the bbox of the nonzero
     pixels; repeat to 3 channels.  `ritnet`: any callable returning the (1,H,W) label map -- iris_b200.RITnet (the
     segmenter on the device), the reference's RITnet, ... -- default = iris_b200.RITnet() like pipelines.py:133-135; or
-    pass the label map itself as `seg`.
+    pass the label map itself as `seg`.  int64 and uint8 label maps are read as they are (e.g. from
+    `iris_b200.RITnet(label_dtype=torch.uint8)`); other integer dtypes are widened to int64.
     Returns (x (3,h,w) fp32, m (1,h,w) bool, x_min, y_min, x_max, y_max) like the reference."""
     from .utils import _bbox_of
 
@@ -556,7 +557,8 @@ def mask_and_crop_iris(x: torch.Tensor,
 
 def iris_masks_and_bboxes(frames: torch.Tensor, segs: torch.Tensor, glint_threshold: float = 0.8, label: int = 2):
     """Batched form of the mask recipe (data_preprocessing.py:164-185, …2020.py:79-100): frames [B,1,H,W],
-    label maps [B,1,H,W] -> (mask uint8 [B,1,H,W], bbox int32 [B,4]) in one kernel launch."""
+    label maps [B,1,H,W] (int64 or uint8 read as they are, other integer dtypes widened to int64) -> (mask uint8 [B,1,H,W],
+    bbox int32 [B,4]) in one kernel launch."""
     from .utils import _bbox_of
 
     bbox, mask, _ = _bbox_of(frames, seg=segs, label=label, threshold=glint_threshold, want_mask=True)

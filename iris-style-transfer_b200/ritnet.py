@@ -1,4 +1,4 @@
-"""Drop-in for models/ritnet/ritnet.py: `RITnet(...)(x)` -> int64 label map (2 = iris), entirely on the device.
+"""Drop-in for models/ritnet/ritnet.py: `RITnet(...)(x)` -> int64 (or uint8) label map (2 = iris), entirely on the device.
 
 The reference pushes every frame through the CPU (uint8 conversion, cv2.LUT, cv2 CLAHE, ritnet.py:88-98) and runs the
 DenseNet2D one image at a time (…2019.py:155, data_preprocessing.py:165).  Here RITnet_transform is three byte kernels
@@ -60,15 +60,23 @@ def normalize_table_f32() -> np.ndarray:
     return t(np.arange(256, dtype=np.uint8).reshape(16, 16)).reshape(-1).numpy().copy()
 
 
+_LABEL_DTYPES = {torch.int64: 0, torch.uint8: 1}
+
+
 class RITnet(torch.nn.Module):
     """models/ritnet/ritnet.py:8-58.  Same constructor arguments; `state_dict=` (a DenseNet2D state dict) replaces the
-    pickle on disk.  forward(x): x (1,h,w) / (h,w) like the reference, or a batch (B,1,h,w) -> int64 labels (B,h,w)
-    on x's device.  Inference only (the reference freezes the model, ritnet.py:31-34); dropout is the identity."""
+    pickle on disk.  forward(x): x (1,h,w) / (h,w) like the reference, or a batch (B,1,h,w) -> labels (B,h,w) of
+    `label_dtype` on x's device.  `label_dtype=torch.uint8` gives the same values at 1 B per pixel, which the mask / bbox,
+    IoU and landmark kernels read without widening; the default is the reference's int64.  Inference only (the reference
+    freezes the model, ritnet.py:31-34); dropout is the identity."""
 
     def __init__(self, dropout: bool = True, prob: float = 0.2, load_pretrained: bool = True,
                  pretrained_path: str = 'models/weights/ritnet_pretrained.pkl',
-                 state_dict: Optional[Dict[str, torch.Tensor]] = None) -> None:
+                 state_dict: Optional[Dict[str, torch.Tensor]] = None, label_dtype: torch.dtype = torch.int64) -> None:
         super().__init__()
+        if label_dtype not in _LABEL_DTYPES:
+            raise ValueError("RITnet: label_dtype must be torch.int64 or torch.uint8, got %s" % (label_dtype,))
+        self.label_dtype = label_dtype
         if state_dict is None:
             if not load_pretrained:
                 raise ValueError("iris_b200.RITnet is an inference engine: pass `state_dict` or keep load_pretrained=True")
@@ -126,7 +134,8 @@ class RITnet(torch.nn.Module):
         blob, gamma, norm = self._tables(dev)
         with torch.cuda.device(dev):
             ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
-            labels = torch.empty(B, H, W, device=dev, dtype=torch.int64)
+            labels = torch.empty(B, H, W, device=dev, dtype=self.label_dtype)
             logits = torch.empty(B, 4, H, W, device=dev, dtype=torch.float32) if return_logits else None
-            _lib.call("isx_ritnet_forward", x, blob, gamma, norm, ws, labels, logits, B, H, W, _lib.stream_ptr())
+            _lib.call("isx_ritnet_forward_typed", x, blob, gamma, norm, ws, labels, _LABEL_DTYPES[self.label_dtype], logits,
+                      B, H, W, _lib.stream_ptr())
         return (labels, logits) if return_logits else labels

@@ -201,9 +201,13 @@ def style_features(style_feats: Sequence[torch.Tensor]) -> torch.Tensor:
     return torch.cat(out, dim=1)
 
 
+_SEG_DTYPES = {torch.int64: 0, torch.uint8: 1}    # label-map dtypes the mask / bbox and IoU kernels read natively
+
+
 def _bbox_of(image: torch.Tensor, seg: Optional[torch.Tensor] = None, label: int = 2,
              threshold: Optional[float] = None, want_mask: bool = False, want_masked: bool = False):
-    """isx_mask_bbox on a batch [B,1,H,W]: returns (bbox int32 [B,4] on device, mask or None, x*m or None)."""
+    """isx_mask_bbox_typed on a batch [B,1,H,W]: returns (bbox int32 [B,4] on device, mask or None, x*m or None).  int64 and
+    uint8 label maps are read as they are; any other dtype is widened to int64 first."""
     if not image.is_cuda:
         raise _lib.IsxError("iris_b200 needs CUDA tensors (B200); there is no CPU path")
     x = image.detach().to(torch.float32).contiguous()
@@ -211,9 +215,12 @@ def _bbox_of(image: torch.Tensor, seg: Optional[torch.Tensor] = None, label: int
     bbox = torch.empty(B, 4, device=x.device, dtype=torch.int32)
     mask = torch.empty(B, 1, H, W, device=x.device, dtype=torch.uint8) if want_mask else None
     xm = torch.empty_like(x) if want_masked else None
-    segc = seg.detach().to(x.device, torch.int64).contiguous() if seg is not None else None
+    segc = None
+    if seg is not None:
+        segc = seg.detach().to(x.device, seg.dtype if seg.dtype in _SEG_DTYPES else torch.int64).contiguous()
     with torch.cuda.device(x.device):
-        _lib.call("isx_mask_bbox", x, segc, int(label), int(threshold is not None),
+        _lib.call("isx_mask_bbox_typed", x, segc, _SEG_DTYPES[segc.dtype] if segc is not None else 0, int(label),
+                  int(threshold is not None),
                   _lib.f32(threshold if threshold is not None else 0.0), mask, xm, bbox, B, H, W, _lib.stream_ptr())
     return bbox, mask, xm
 
@@ -238,21 +245,24 @@ def crop_image(image: torch.Tensor, return_idx: bool = False):
 
 def cal_IoUs(preds: torch.Tensor, targets: torch.Tensor, num_class: int = 4, eps: float = 1e-6, device="cuda:0"):
     """utils.py:163-194: IoU per image and class and their mean for label maps of shape (b, h, w).  One fused pass over the
-    two maps (`isx_seg_iou`: ballots + popc, exact counts) instead of the reference's ~30 elementwise passes; returns
-    (iou_per_class: list of num_class tensors [b], miou [b]) on the device, bit-identical to the reference."""
+    two maps (`isx_seg_iou_typed`: exact counts) instead of the reference's ~30 elementwise passes; returns
+    (iou_per_class: list of num_class tensors [b], miou [b]) on the device, bit-identical to the reference.  Two uint8 maps
+    are read as they are (2 B per pixel); any other combination, mixed dtypes included, is widened to int64 first, so a
+    value >= 256 in an int64 map keeps meaning "no class"."""
     if preds.shape != targets.shape:      # the reference broadcasts (data_preprocessing.py:168 passes (1,h,w) vs (1,h,w))
         preds, targets = torch.broadcast_tensors(preds, targets)
     if preds.dim() != 3:
         raise ValueError("label maps must be (b, h, w), got %s" % (tuple(preds.shape),))
     dev = preds.device if preds.is_cuda else (targets.device if targets.is_cuda else torch.device(device))
-    p = preds.detach().to(dev, torch.int64).contiguous()
-    t = targets.detach().to(dev, torch.int64).contiguous()
+    dt = torch.uint8 if preds.dtype == targets.dtype == torch.uint8 else torch.int64
+    p = preds.detach().to(dev, dt).contiguous()
+    t = targets.detach().to(dev, dt).contiguous()
     B, H, W = p.shape
     with torch.cuda.device(dev):
         counts = torch.empty(B, num_class, 2, device=dev, dtype=torch.int32)
         iou = torch.empty(B, num_class, device=dev, dtype=torch.float32)
         miou = torch.empty(B, device=dev, dtype=torch.float32)
-        _lib.call("isx_seg_iou", p, t, B, _lib.i64(H * W), int(num_class), _lib.f32(eps), counts, iou, miou, _lib.stream_ptr())
+        _lib.call("isx_seg_iou_typed", p, t, _SEG_DTYPES[dt], B, _lib.i64(H * W), int(num_class), _lib.f32(eps), counts, iou, miou, _lib.stream_ptr())
     return [iou[:, c] for c in range(num_class)], miou
 
 
