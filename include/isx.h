@@ -207,6 +207,12 @@ int isx_lbfgs_tick(float* x, const float* grad, float* grad_prev, void* S, void*
                    void* scratch, const double* loss_c, const double* loss_s, int images_per_problem, int P,
                    int64_t N, const isx_lbfgs_config* cfg, double* hist_c, double* hist_s, int tick,
                    isx_stream stream);
+/* isx_lbfgs_tick with per-problem loss weights: problem p's loss (its tolerance_change test) is
+ * c_weight[p] * c_p + s_weight[p] * s_p with c_weight / s_weight device double [P]; cfg->c_weight / s_weight are not read. */
+int isx_lbfgs_tick_problems(float* x, const float* grad, float* grad_prev, void* S, void* Y, void* state, void* mats,
+                            void* scratch, const double* loss_c, const double* loss_s, int images_per_problem, int P,
+                            int64_t N, const isx_lbfgs_config* cfg, const double* c_weight, const double* s_weight,
+                            double* hist_c, double* hist_s, int tick, isx_stream stream);
 /* done_out[p] (device int32) <- number of closure evaluations problem p performed once it has finished its
  * pipelines.py:79 loop, 0 while it is still running */
 int isx_lbfgs_done_flags(const void* state, int P, int32_t* done_out, isx_stream stream);
@@ -286,6 +292,22 @@ int isx_nst_style_features(const isx_nst_config* cfg, const isx_nst_buffers* buf
 /* closure evaluation: loss_c/loss_s double [B] (unweighted, per image), grad fp32 [B,xc,H,W] = d(alpha c + beta s)/dx */
 int isx_nst_eval(const isx_nst_config* cfg, const isx_nst_buffers* bufs, const float* x, double* loss_c,
                  double* loss_s, float* grad, isx_stream stream);
+
+/* ---- several coupled problems in one batch: P = B / g problems of g images each (nst(problem_size=g)) ---------------
+ * Problem p is the images [p*g, (p+1)*g): its content loss is the mean over its g images, its style loss the sum, and it
+ * has its own alpha / beta.  The weights are read from device memory on every call, so a captured tick stays valid. */
+typedef struct {
+  int32_t images_per_problem;           /* g >= 1, B % g == 0 */
+  int32_t style_target_b;               /* 1, P or B: image b reads style target b / (B / style_target_b); replaces
+                                           cfg->style_target_b */
+  const double* c_weight;               /* device [P]: alpha of each problem (cfg->c_weight is not read) */
+  const double* s_weight;               /* device [P]: beta of each problem (cfg->s_weight is not read) */
+} isx_nst_problems;
+/* isx_nst_eval for P problems: same outputs (per-image unweighted losses), grad = d(sum_p alpha_p c_p + beta_p s_p)/dx.
+ * cfg->coupled is not read.  With g = B, style_target_b in {1, B} and equal weights this is isx_nst_eval with coupled = 1,
+ * with g = 1 isx_nst_eval with coupled = 0, bit for bit. */
+int isx_nst_eval_problems(const isx_nst_config* cfg, const isx_nst_buffers* bufs, const isx_nst_problems* problems,
+                          const float* x, double* loss_c, double* loss_s, float* grad, isx_stream stream);
 
 /* ---- K10: iris mask + bounding box (pipelines.py:139-165 mask_and_crop_iris; utils.py:44-72 crop_image) --
  * x fp32 [B,1,H,W]; seg int64 [B,1,H,W] label map or NULL; m = (seg == label) & (x <= threshold) (either

@@ -490,10 +490,15 @@ int tap_add_mask(const __nv_bfloat16* g, const __nv_bfloat16* add, const float* 
 //   D[b]    = grad_scale * (G - T)  in bf16, full     (dF = D . F, see conv_tc 1x1 mode)
 //   triu    (optional) upper triangle incl. diagonal in torch.triu_indices order, row b at triu + b * triu_ld
 // ------------------------------------------------------------------------------------------
+//   kPerProblem: image b belongs to problem b / pw.ipp, its gradient scale is (float)(pw.weight[b / pw.ipp] * pw.k1 * pw.k2)
+//                (beta_p * w_l * inv_n, the same double products the host forms for the scalar grad_scale) and its target
+//                is target[b / pw.target_div]
+template <bool kPerProblem>
 __global__ void __launch_bounds__(256)
 gram_finalize_kernel(const float* __restrict__ partial, int splits, int C, float inv_n, float* __restrict__ G_out,
                      const float* __restrict__ target, int target_b, double loss_scale, double* __restrict__ loss,
-                     float grad_scale, __nv_bfloat16* __restrict__ D_out, float* __restrict__ triu, long triu_ld) {
+                     float grad_scale, __nv_bfloat16* __restrict__ D_out, float* __restrict__ triu, long triu_ld,
+                     ProblemWeights pw) {
   __shared__ float sg[32][33];
   __shared__ double red[8];
   const int b = blockIdx.y;
@@ -505,7 +510,8 @@ gram_finalize_kernel(const float* __restrict__ partial, int splits, int C, float
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const long cc = static_cast<long>(C) * C;
   const float* pb = partial + static_cast<long>(b) * splits * cc;
-  const float* tb = target ? target + (target_b > 1 ? b : 0) * cc : nullptr;
+  const float* tb = target ? target + (kPerProblem ? b / pw.target_div : (target_b > 1 ? b : 0)) * cc : nullptr;
+  if (kPerProblem) grad_scale = static_cast<float>(pw.weight[b / pw.ipp] * pw.k1 * pw.k2);
   float d2 = 0.f;
   float g[4];
 #pragma unroll
@@ -553,12 +559,16 @@ gram_finalize_kernel(const float* __restrict__ partial, int splits, int C, float
 
 int gram_finalize(const float* partial, int B, int splits, int C, float inv_n, float* G_out, const float* target,
                   int target_b, double loss_scale, double* loss, float grad_scale, __nv_bfloat16* D_out,
-                  cudaStream_t s, float* triu, long triu_ld) {
+                  cudaStream_t s, float* triu, long triu_ld, const ProblemWeights* pw) {
   ISX_REQUIRE(C % 32 == 0, "gram_finalize: C = %d must be a multiple of 32", C);
   const int nt = C / 32;
   dim3 grid(static_cast<unsigned>(nt * (nt + 1) / 2), B);
-  gram_finalize_kernel<<<grid, 256, 0, s>>>(partial, splits, C, inv_n, G_out, target, target_b, loss_scale,
-                                            target ? loss : nullptr, grad_scale, D_out, triu, triu_ld);
+  if (pw)
+    gram_finalize_kernel<true><<<grid, 256, 0, s>>>(partial, splits, C, inv_n, G_out, target, target_b, loss_scale,
+                                                    target ? loss : nullptr, grad_scale, D_out, triu, triu_ld, *pw);
+  else
+    gram_finalize_kernel<false><<<grid, 256, 0, s>>>(partial, splits, C, inv_n, G_out, target, target_b, loss_scale,
+                                                     target ? loss : nullptr, grad_scale, D_out, triu, triu_ld, ProblemWeights());
   ISX_LAUNCH_CHECK();
   return 0;
 }
@@ -567,11 +577,14 @@ int gram_finalize(const float* partial, int B, int splits, int C, float inv_n, f
 // Content loss (ContentLoss_L2, utils.py:285-290): loss[b] += loss_scale * sum((p-t)^2);
 // grad = grad_scale * (p - t) * (p > 0)  (dL/d relu-output, already pushed through the ReLU)
 // ------------------------------------------------------------------------------------------
+// kPerProblem: grad_scale of image b = (float)(pw.weight[b / pw.ipp] * pw.k1 / pw.k2)  (alpha_p * content_w / denom)
+template <bool kPerProblem>
 __global__ void __launch_bounds__(256)
 content_mse_kernel(const __nv_bfloat16* __restrict__ pred, const __nv_bfloat16* __restrict__ target, int target_b,
                    __nv_bfloat16* __restrict__ grad, long per_image8, double loss_scale, float grad_scale,
-                   double* __restrict__ loss, int relu_mask) {
+                   double* __restrict__ loss, int relu_mask, ProblemWeights pw) {
   const int b = blockIdx.y;
+  if (kPerProblem) grad_scale = static_cast<float>(pw.weight[b / pw.ipp] * pw.k1 / pw.k2);
   const uint4* p = reinterpret_cast<const uint4*>(pred) + b * per_image8;
   const uint4* t = reinterpret_cast<const uint4*>(target) + (target_b > 1 ? b : 0) * per_image8;
   uint4* g = grad ? reinterpret_cast<uint4*>(grad) + b * per_image8 : nullptr;
@@ -601,12 +614,17 @@ content_mse_kernel(const __nv_bfloat16* __restrict__ pred, const __nv_bfloat16* 
 }
 
 int content_mse(const __nv_bfloat16* pred, const __nv_bfloat16* target, int target_b, __nv_bfloat16* grad, int B,
-                long per_image, double loss_scale, float grad_scale, double* loss, cudaStream_t s, int relu_mask) {
+                long per_image, double loss_scale, float grad_scale, double* loss, cudaStream_t s, int relu_mask,
+                const ProblemWeights* pw) {
   ISX_REQUIRE(per_image % 8 == 0, "content_mse: per-image size %ld not a multiple of 8", per_image);
   const long n8 = per_image / 8;
   int bx = static_cast<int>(std::min<long>((n8 + 255) / 256, static_cast<long>(isx_num_sms()) * 8 / std::max(1, std::min(B, 8)) + 1));
   dim3 grid(bx, B);
-  content_mse_kernel<<<grid, 256, 0, s>>>(pred, target, target_b, grad, n8, loss_scale, grad_scale, loss, relu_mask);
+  if (pw)
+    content_mse_kernel<true><<<grid, 256, 0, s>>>(pred, target, target_b, grad, n8, loss_scale, grad_scale, loss, relu_mask, *pw);
+  else
+    content_mse_kernel<false><<<grid, 256, 0, s>>>(pred, target, target_b, grad, n8, loss_scale, grad_scale, loss, relu_mask,
+                                                   ProblemWeights());
   ISX_LAUNCH_CHECK();
   return 0;
 }
@@ -671,12 +689,15 @@ int chan_sums(const __nv_bfloat16* f, int B, long HW, int C, double* sums, cudaS
 //   loss[b] += loss_scale * sum_c[(mu-mu_t)^2 + (sd-sd_t)^2]            (loss_scale = w_l / C)
 //   dL/dF[p,c] = aff_a[b,c] + aff_b[b,c] * F[p,c]   with (grad_scale = beta * w_l / C)
 //     aff_b = grad_scale * 2 (sd - sd_t) / ((n-1) sd),  aff_a = grad_scale * 2 (mu - mu_t) / n - aff_b * mu
+// kPerProblem: grad_scale of image b = pw.weight[b / pw.ipp] * pw.k1 / pw.k2  (beta_p * w_l / C), target b / pw.target_div
+template <bool kPerProblem>
 __global__ void bn_finalize_kernel(const double* __restrict__ sums, int B, int C, double n, float* __restrict__ mean,
                                    float* __restrict__ stdv, const float* __restrict__ t_mean,
                                    const float* __restrict__ t_std, int target_b, double loss_scale, double grad_scale,
                                    double* __restrict__ loss, float* __restrict__ aff_a, float* __restrict__ aff_b,
-                                   long out_ld) {
+                                   long out_ld, ProblemWeights pw) {
   const int b = blockIdx.x;
+  if (kPerProblem) grad_scale = pw.weight[b / pw.ipp] * pw.k1 / pw.k2;
   double lacc = 0.0;
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
     const double s1 = sums[(static_cast<long>(b) * C + c) * 2], s2 = sums[(static_cast<long>(b) * C + c) * 2 + 1];
@@ -687,7 +708,7 @@ __global__ void bn_finalize_kernel(const double* __restrict__ sums, int B, int C
     if (mean) mean[b * out_ld + c] = static_cast<float>(mu);
     if (stdv) stdv[b * out_ld + c] = static_cast<float>(sd);
     if (t_mean) {
-      const int tb = target_b > 1 ? b : 0;
+      const int tb = kPerProblem ? b / pw.target_div : (target_b > 1 ? b : 0);
       const double dm = static_cast<double>(static_cast<float>(mu)) - t_mean[tb * C + c];
       const double ds = static_cast<double>(static_cast<float>(sd)) - t_std[tb * C + c];
       lacc += dm * dm + ds * ds;
@@ -739,9 +760,14 @@ int stats_from_gram(const float* partial, const float* csum, int B, int splits, 
 
 int bn_finalize(const double* sums, int B, int C, long HW, float* mean, float* stdv, const float* t_mean,
                 const float* t_std, int target_b, double loss_scale, double grad_scale, double* loss, float* aff_a,
-                float* aff_b, cudaStream_t s, long out_ld) {
-  bn_finalize_kernel<<<B, 256, 0, s>>>(sums, B, C, static_cast<double>(HW), mean, stdv, t_mean, t_std, target_b,
-                                       loss_scale, grad_scale, loss, aff_a, aff_b, out_ld > 0 ? out_ld : C);
+                float* aff_b, cudaStream_t s, long out_ld, const ProblemWeights* pw) {
+  if (pw)
+    bn_finalize_kernel<true><<<B, 256, 0, s>>>(sums, B, C, static_cast<double>(HW), mean, stdv, t_mean, t_std, target_b,
+                                               loss_scale, grad_scale, loss, aff_a, aff_b, out_ld > 0 ? out_ld : C, *pw);
+  else
+    bn_finalize_kernel<false><<<B, 256, 0, s>>>(sums, B, C, static_cast<double>(HW), mean, stdv, t_mean, t_std, target_b,
+                                                loss_scale, grad_scale, loss, aff_a, aff_b, out_ld > 0 ? out_ld : C,
+                                                ProblemWeights());
   ISX_LAUNCH_CHECK();
   return 0;
 }

@@ -27,11 +27,21 @@ int tap_add_mask(const __nv_bfloat16* g, const __nv_bfloat16* add, const float* 
 int mask_features(const __nv_bfloat16* f, const float* m, int mask_b, __nv_bfloat16* fm, __nv_bfloat16* fm2, int B,
                   long HW, int C, cudaStream_t s);
 int avgpool2x2_f32(const float* in, float* out, int B, int H, int W, cudaStream_t s);
+// Several coupled problems in one batch (isx_nst_eval_problems): image b belongs to problem b / ipp and scales its loss
+// gradient by that problem's weight.  Each finalize kernel forms the scale from weight[p], k1 and k2 with the same double
+// operations the host uses for its scalar grad_scale, so that one problem's images match a scalar call bit for bit.
+struct ProblemWeights {
+  const double* weight = nullptr;  // device [P]: alpha (content) or beta (style) per problem
+  int ipp = 1;                     // images per problem
+  int target_div = 1;              // image b reads style target b / target_div (B / style target batch)
+  double k1 = 0.0, k2 = 0.0;
+};
 int gram_finalize(const float* partial, int B, int splits, int C, float inv_n, float* G_out, const float* target,
                   int target_b, double loss_scale, double* loss, float grad_scale, __nv_bfloat16* D_out,
-                  cudaStream_t s, float* triu = nullptr, long triu_ld = 0);
+                  cudaStream_t s, float* triu = nullptr, long triu_ld = 0, const ProblemWeights* pw = nullptr);
 int content_mse(const __nv_bfloat16* pred, const __nv_bfloat16* target, int target_b, __nv_bfloat16* grad, int B,
-                long per_image, double loss_scale, float grad_scale, double* loss, cudaStream_t s, int relu_mask = 1);
+                long per_image, double loss_scale, float grad_scale, double* loss, cudaStream_t s, int relu_mask = 1,
+                const ProblemWeights* pw = nullptr);
 int chan_sums(const __nv_bfloat16* f, int B, long HW, int C, double* sums, cudaStream_t s, const float* mask = nullptr,
               int mask_b = 0);
 int masked_affine_grad(const __nv_bfloat16* f, const float* m, int mask_b, const float* aff_a, const float* aff_b,
@@ -40,6 +50,7 @@ int stats_from_gram(const float* partial, const float* csum, int B, int splits, 
                     long out_ld, cudaStream_t s);
 int bn_finalize(const double* sums, int B, int C, long HW, float* mean, float* stdv, const float* t_mean,
                 const float* t_std, int target_b, double loss_scale, double grad_scale, double* loss, float* aff_a,
-                float* aff_b, cudaStream_t s, long out_ld = 0);  // out_ld: row stride of mean / stdv (0 = C)
+                float* aff_b, cudaStream_t s, long out_ld = 0,   // out_ld: row stride of mean / stdv (0 = C)
+                const ProblemWeights* pw = nullptr);
 
 }  // namespace isx

@@ -220,11 +220,14 @@ __device__ __forceinline__ double block_sum_128(double v, double* red) {
   return red[0] + red[1] + red[2] + red[3];
 }
 
+// kPerProblem: the loss weights of problem p are c_w[p], s_w[p] (device arrays) instead of cfg.c_weight, cfg.s_weight
+template <bool kPerProblem>
 __global__ void __launch_bounds__(128)
 lbfgs_control_kernel(LbfgsState* __restrict__ states, double* __restrict__ mats, const double* __restrict__ dots,
                      const double* __restrict__ loss_c,
                      const double* __restrict__ loss_s, int images_per_problem, int M1, LbfgsConfig cfg,
-                     double* __restrict__ hist_c, double* __restrict__ hist_s, int tick, int P) {
+                     double* __restrict__ hist_c, double* __restrict__ hist_s, int tick, int P,
+                     const double* __restrict__ c_w, const double* __restrict__ s_w) {
   const int p = blockIdx.x;
   LbfgsState& st = states[p];
   __shared__ double red[4];
@@ -265,7 +268,8 @@ lbfgs_control_kernel(LbfgsState* __restrict__ states, double* __restrict__ mats,
 
   // ---- state machine (lbfgs.py:364-374, 388-392, 504-526) ----
   if (tid == 0) {
-    const double loss = cfg.c_weight * lc + cfg.s_weight * ls;
+    const double cw = kPerProblem ? c_w[p] : cfg.c_weight, sw = kPerProblem ? s_w[p] : cfg.s_weight;
+    const double loss = cw * lc + sw * ls;
     st.last_c = lc; st.last_s = ls;
     hist_c[static_cast<long>(st.func_evals) * P + p] = lc;
     hist_s[static_cast<long>(st.func_evals) * P + p] = ls;
@@ -523,7 +527,8 @@ int clamp01(float* x, long n, cudaStream_t s) {
 
 int lbfgs_tick(float* x, const float* g, float* g_prev, void* S, void* Y, int history_bf16, LbfgsState* states, double* mats,
                float* part, float* ext, double* dots, const double* loss_c, const double* loss_s, int images_per_problem, int P,
-               long N, const LbfgsConfig& cfg, double* hist_c, double* hist_s, int tick, cudaStream_t s) {
+               long N, const LbfgsConfig& cfg, double* hist_c, double* hist_s, int tick, cudaStream_t s, const double* c_w,
+               const double* s_w) {
   const int M1 = cfg.history + 1;
   ISX_REQUIRE(M1 <= kMaxSlots, "lbfgs: history %d exceeds %d", cfg.history, kMaxSlots - 1);
   const int nblk = lbfgs_nblk(N);
@@ -539,8 +544,12 @@ int lbfgs_tick(float* x, const float* g, float* g_prev, void* S, void* Y, int hi
   ISX_LAUNCH_CHECK();
   lbfgs_reduce_kernel<<<dim3(M1 + 1, P), 128, 0, s>>>(states, part, ext, M1, nblk, dots);
   ISX_LAUNCH_CHECK();
-  lbfgs_control_kernel<<<P, 128, 0, s>>>(states, mats, dots, loss_c, loss_s, images_per_problem, M1, cfg, hist_c, hist_s,
-                                         tick, P);
+  if (c_w)
+    lbfgs_control_kernel<true><<<P, 128, 0, s>>>(states, mats, dots, loss_c, loss_s, images_per_problem, M1, cfg, hist_c,
+                                                 hist_s, tick, P, c_w, s_w);
+  else
+    lbfgs_control_kernel<false><<<P, 128, 0, s>>>(states, mats, dots, loss_c, loss_s, images_per_problem, M1, cfg, hist_c,
+                                                  hist_s, tick, P, nullptr, nullptr);
   ISX_LAUNCH_CHECK();
   if (history_bf16)
     lbfgs_update_kernel<__nv_bfloat16><<<grid, kDotThreads, 0, s>>>(x, g, g_prev, static_cast<__nv_bfloat16*>(S),

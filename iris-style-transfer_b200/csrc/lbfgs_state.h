@@ -42,6 +42,7 @@ int clamp01(float* x, long n, cudaStream_t s);
 int lbfgs_tick(float* x, const float* g, float* g_prev, void* S, void* Y, int history_bf16, LbfgsState* states,
                double* mats,
                float* part, float* ext, double* dots, const double* loss_c, const double* loss_s, int images_per_problem, int P,
-               long N, const LbfgsConfig& cfg, double* hist_c, double* hist_s, int tick, cudaStream_t s);
+               long N, const LbfgsConfig& cfg, double* hist_c, double* hist_s, int tick, cudaStream_t s,
+               const double* c_w = nullptr, const double* s_w = nullptr);  // per-problem alpha / beta (device [P]) or cfg's
 
 }  // namespace isx

@@ -362,11 +362,12 @@ int run_backward(const isx_nst_config* c, const isx_nst_buffers* b, const Layout
 }
 }  // namespace
 
-extern "C" int isx_nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const float* x, double* loss_c,
-                            double* loss_s, float* grad, isx_stream stream) {
-  ISX_REQUIRE(c && b && x && loss_c && loss_s && grad && b->workspace, "isx_nst_eval: null pointer");
-  ISX_REQUIRE(c->n_style + c->n_content > 0, "isx_nst_eval: no loss taps");
-  ISX_REQUIRE(c->style_mask_b == 0 || c->style_mask_b == 1 || c->style_mask_b == c->B, "isx_nst_eval: style mask batch %d", c->style_mask_b);
+namespace {
+// One closure evaluation.  pr == nullptr: the batch is one problem (c->coupled) or B problems, with the scalar weights of
+// c.  Otherwise the batch is B / g problems of g images, each with its own alpha / beta (device arrays) and the style
+// target of image b at b / (B / pr->style_target_b); the arguments were validated by isx_nst_eval_problems.
+int nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_problems* pr, const float* x, double* loss_c,
+             double* loss_s, float* grad, isx_stream stream) {
   Layout L;
   if (int rc = make_layout(c, &L)) return rc;
   cudaStream_t s = S(stream);
@@ -377,6 +378,15 @@ extern "C" int isx_nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, c
               "isx_nst_eval: conv %d is not tapped", deepest);
   ISX_CHECK_CUDA(cudaMemsetAsync(loss_c, 0, sizeof(double) * B, s));
   ISX_CHECK_CUDA(cudaMemsetAsync(loss_s, 0, sizeof(double) * B, s));
+  // per-problem beta of the style taps: the finalize kernels form beta_p * w * k2 (Gram) or beta_p * w / k2 (BN)
+  auto style_weights = [&](double w, double k2) {
+    ProblemWeights pw;
+    if (pr) {
+      pw.weight = pr->s_weight; pw.ipp = pr->images_per_problem; pw.target_div = B / pr->style_target_b;
+      pw.k1 = w; pw.k2 = k2;
+    }
+    return pw;
+  };
 
   // losses of everything tapped at `id` (a conv's ReLU output or a pool output), evaluated on the stored activation
   auto tap_losses = [&](int id) -> int {
@@ -400,8 +410,10 @@ extern "C" int isx_nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, c
         const int splits = gram_pick_splits(B, static_cast<int>(HW), C);
         int rc = gram_sym_partial(act, B, static_cast<int>(HW), C, splits, atf(b, L.gram_ws), c->style_mask_b > 0 ? &gm : nullptr, s);
         if (rc) return rc;
+        const ProblemWeights pw = style_weights(w, inv_n);
         rc = gram_finalize(atf(b, L.gram_ws), B, splits, C, static_cast<float>(inv_n), nullptr, b->gram_target[st],
-                           c->style_target_b, 0.25 * w, loss_s, static_cast<float>(c->s_weight * w * inv_n), at(b, L.D[st]), s);
+                           c->style_target_b, 0.25 * w, loss_s, static_cast<float>(c->s_weight * w * inv_n), at(b, L.D[st]), s,
+                           nullptr, 0, pr ? &pw : nullptr);
         if (rc) return rc;
       } else {  // StyleLoss_BN (utils.py:350-355)
         ISX_REQUIRE(b->bn_target_mean[st] && b->bn_target_std[st], "nst: BN target %d missing", st);
@@ -415,8 +427,10 @@ extern "C" int isx_nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, c
         }
         int rc = chan_sums(act, B, HW, C, sums, s, m, c->style_mask_b);
         if (rc) return rc;
+        const ProblemWeights pw = style_weights(w, static_cast<double>(C));
         rc = bn_finalize(sums, B, C, HW, nullptr, nullptr, b->bn_target_mean[st], b->bn_target_std[st],
-                         c->style_target_b, w / C, c->s_weight * w / C, loss_s, atf(b, L.aff_a[st]), atf(b, L.aff_b[st]), s);
+                         c->style_target_b, w / C, c->s_weight * w / C, loss_s, atf(b, L.aff_a[st]), atf(b, L.aff_b[st]), s,
+                         0, pr ? &pw : nullptr);
         if (rc) return rc;
         if (m)  // the gradient is no longer affine in F alone: m a + m^2 b F, materialised as a gradient map (buffer fm2)
           if (int rc2 = masked_affine_grad(act, m, c->style_mask_b, atf(b, L.aff_a[st]), atf(b, L.aff_b[st]), at(b, L.fm2[st]), B, HW, C, s)) return rc2;
@@ -426,10 +440,13 @@ extern "C" int isx_nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, c
     if (ct >= 0) {  // ContentLoss_L2 (utils.py:285-290): 0.5 * w * mean((p-t)^2)
       ISX_REQUIRE(b->content_target[ct], "nst: content target %d missing", ct);
       const long per_image = HW * C;
-      const double denom = static_cast<double>(per_image) * (c->coupled ? B : 1);
+      // F.mse_loss over the problem's batch: B images when coupled, g with several problems, else one
+      const double denom = static_cast<double>(per_image) * (pr ? pr->images_per_problem : c->coupled ? B : 1);
+      ProblemWeights pw;
+      if (pr) { pw.weight = pr->c_weight; pw.ipp = pr->images_per_problem; pw.k1 = c->content_w[ct]; pw.k2 = denom; }
       int rc = content_mse(act, reinterpret_cast<const bf16*>(b->content_target[ct]), c->content_target_b,
                            at(b, L.cgrad[ct]), B, per_image, 0.5 * c->content_w[ct] / denom,
-                           static_cast<float>(c->c_weight * c->content_w[ct] / denom), loss_c, s);
+                           static_cast<float>(c->c_weight * c->content_w[ct] / denom), loss_c, s, 1, pr ? &pw : nullptr);
       if (rc) return rc;
     }
     return 0;
@@ -467,6 +484,33 @@ extern "C" int isx_nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, c
     }
   }
   return run_backward(c, b, L, src, nullptr, grad, s);
+}
+}  // namespace
+
+extern "C" int isx_nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const float* x, double* loss_c,
+                            double* loss_s, float* grad, isx_stream stream) {
+  ISX_REQUIRE(c && b && x && loss_c && loss_s && grad && b->workspace, "isx_nst_eval: null pointer");
+  ISX_REQUIRE(c->n_style + c->n_content > 0, "isx_nst_eval: no loss taps");
+  ISX_REQUIRE(c->style_mask_b == 0 || c->style_mask_b == 1 || c->style_mask_b == c->B, "isx_nst_eval: style mask batch %d", c->style_mask_b);
+  return nst_eval(c, b, nullptr, x, loss_c, loss_s, grad, stream);
+}
+
+extern "C" int isx_nst_eval_problems(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_problems* pr,
+                                     const float* x, double* loss_c, double* loss_s, float* grad, isx_stream stream) {
+  ISX_REQUIRE(c && b && pr && x && loss_c && loss_s && grad && b->workspace, "isx_nst_eval_problems: null pointer");
+  ISX_REQUIRE(c->n_style + c->n_content > 0, "isx_nst_eval_problems: no loss taps");
+  const int B = c->B, g = pr->images_per_problem;
+  ISX_REQUIRE(B > 0 && g >= 1 && B % g == 0, "isx_nst_eval_problems: batch %d is not a whole number of problems of %d images",
+              B, g);
+  const int P = B / g, tb = pr->style_target_b;
+  ISX_REQUIRE(c->n_style == 0 || tb == 1 || tb == P || tb == B,
+              "isx_nst_eval_problems: style target batch %d must be 1, %d (problems) or %d (images)", tb, P, B);
+  ISX_REQUIRE(pr->c_weight && pr->s_weight, "isx_nst_eval_problems: null per-problem weight array");
+  ISX_REQUIRE(c->style_mask_b == 0 || c->style_mask_b == 1 || c->style_mask_b == B,
+              "isx_nst_eval_problems: style mask batch %d", c->style_mask_b);
+  isx_nst_problems q = *pr;
+  if (c->n_style == 0) q.style_target_b = B;   // no target is read
+  return nst_eval(c, b, &q, x, loss_c, loss_s, grad, stream);
 }
 
 extern "C" int isx_nst_prepare_style_masks(const isx_nst_config* c, const isx_nst_buffers* b, isx_stream stream) {
@@ -570,13 +614,11 @@ extern "C" int isx_lbfgs_init(void* state, int P, isx_stream stream) {
   ISX_REQUIRE(state && P > 0, "isx_lbfgs_init: bad arguments");
   return lbfgs_init(static_cast<LbfgsState*>(state), P, S(stream));
 }
-extern "C" int isx_lbfgs_tick(float* x, const float* grad, float* grad_prev, void* Sh, void* Yh, void* state,
-                              void* mats, void* scratch, const double* loss_c, const double* loss_s,
-                              int images_per_problem, int P, int64_t N, const isx_lbfgs_config* cfg, double* hist_c,
-                              double* hist_s, int tick, isx_stream stream) {
-  ISX_REQUIRE(x && grad && grad_prev && Sh && Yh && state && mats && scratch && loss_c && loss_s && cfg && hist_c && hist_s,
-              "isx_lbfgs_tick: null pointer");
-  ISX_REQUIRE(cfg->history >= 1 && cfg->history <= 100, "isx_lbfgs_tick: history %d must be in 1..100", cfg->history);
+namespace {
+int lbfgs_tick_impl(float* x, const float* grad, float* grad_prev, void* Sh, void* Yh, void* state, void* mats, void* scratch,
+                    const double* loss_c, const double* loss_s, int images_per_problem, int P, int64_t N,
+                    const isx_lbfgs_config* cfg, const double* c_weight, const double* s_weight, double* hist_c,
+                    double* hist_s, int tick, isx_stream stream) {
   LbfgsConfig lc;
   lc.epochs = cfg->epochs; lc.max_iter = cfg->max_iter; lc.max_eval = cfg->max_eval; lc.history = cfg->history;
   lc.lr = cfg->lr; lc.tolerance_grad = cfg->tolerance_grad; lc.tolerance_change = cfg->tolerance_change;
@@ -587,7 +629,35 @@ extern "C" int isx_lbfgs_tick(float* x, const float* grad, float* grad_prev, voi
   const int64_t floats = static_cast<int64_t>(P) * nblk * (static_cast<int64_t>(cfg->history + 1) * 4 + 4);
   double* dots = reinterpret_cast<double*>(static_cast<char*>(scratch) + ((floats * 4 + 255) / 256) * 256);
   return lbfgs_tick(x, grad, grad_prev, Sh, Yh, cfg->history_bf16, static_cast<LbfgsState*>(state), static_cast<double*>(mats), part, ext,
-                    dots, loss_c, loss_s, images_per_problem, P, N, lc, hist_c, hist_s, tick, S(stream));
+                    dots, loss_c, loss_s, images_per_problem, P, N, lc, hist_c, hist_s, tick, S(stream), c_weight, s_weight);
+}
+}  // namespace
+
+extern "C" int isx_lbfgs_tick(float* x, const float* grad, float* grad_prev, void* Sh, void* Yh, void* state,
+                              void* mats, void* scratch, const double* loss_c, const double* loss_s,
+                              int images_per_problem, int P, int64_t N, const isx_lbfgs_config* cfg, double* hist_c,
+                              double* hist_s, int tick, isx_stream stream) {
+  ISX_REQUIRE(x && grad && grad_prev && Sh && Yh && state && mats && scratch && loss_c && loss_s && cfg && hist_c && hist_s,
+              "isx_lbfgs_tick: null pointer");
+  ISX_REQUIRE(cfg->history >= 1 && cfg->history <= 100, "isx_lbfgs_tick: history %d must be in 1..100", cfg->history);
+  return lbfgs_tick_impl(x, grad, grad_prev, Sh, Yh, state, mats, scratch, loss_c, loss_s, images_per_problem, P, N, cfg,
+                         nullptr, nullptr, hist_c, hist_s, tick, stream);
+}
+
+extern "C" int isx_lbfgs_tick_problems(float* x, const float* grad, float* grad_prev, void* Sh, void* Yh, void* state,
+                                       void* mats, void* scratch, const double* loss_c, const double* loss_s,
+                                       int images_per_problem, int P, int64_t N, const isx_lbfgs_config* cfg,
+                                       const double* c_weight, const double* s_weight, double* hist_c, double* hist_s,
+                                       int tick, isx_stream stream) {
+  ISX_REQUIRE(x && grad && grad_prev && Sh && Yh && state && mats && scratch && loss_c && loss_s && cfg && hist_c && hist_s,
+              "isx_lbfgs_tick_problems: null pointer");
+  ISX_REQUIRE(c_weight && s_weight, "isx_lbfgs_tick_problems: null per-problem weight array");
+  ISX_REQUIRE(images_per_problem >= 1 && P >= 1 && N >= 1, "isx_lbfgs_tick_problems: %d problems of %d images, N = %lld",
+              P, images_per_problem, (long long)N);
+  ISX_REQUIRE(cfg->history >= 1 && cfg->history <= 100, "isx_lbfgs_tick_problems: history %d must be in 1..100",
+              cfg->history);
+  return lbfgs_tick_impl(x, grad, grad_prev, Sh, Yh, state, mats, scratch, loss_c, loss_s, images_per_problem, P, N, cfg,
+                         c_weight, s_weight, hist_c, hist_s, tick, stream);
 }
 
 __global__ void done_flags_kernel(const LbfgsState* st, int P, int32_t* out) {

@@ -83,6 +83,13 @@ class LbfgsConfig(ctypes.Structure):
     ]
 
 
+class NstProblems(ctypes.Structure):
+    _fields_ = [
+        ("images_per_problem", ctypes.c_int32), ("style_target_b", ctypes.c_int32),
+        ("c_weight", ctypes.c_void_p), ("s_weight", ctypes.c_void_p),
+    ]
+
+
 class PackedVGG:
     """VGG-19 conv parameters packed once for the device kernels (isx_pack_conv3x3_weights)."""
 
@@ -162,6 +169,19 @@ class NstEngine:
         self._keep: List[torch.Tensor] = []  # targets referenced by raw pointer
         self.loss_c = torch.zeros(B, device=self.device, dtype=torch.float64)
         self.loss_s = torch.zeros(B, device=self.device, dtype=torch.float64)
+        self.problems: Optional[NstProblems] = None
+
+    def set_problems(self, images_per_problem: int, c_weight: torch.Tensor, s_weight: torch.Tensor):
+        """Evaluate the batch as B / images_per_problem coupled problems (isx_nst_eval_problems) with per-problem alpha /
+        beta: device float64 [P] tensors, read on every eval (they may be updated in place between evals)."""
+        for w in (c_weight, s_weight):
+            assert w.is_cuda and w.dtype == torch.float64 and w.is_contiguous()
+            assert w.shape == (self.cfg.B // images_per_problem,)
+        self._keep += [c_weight, s_weight]
+        pr = NstProblems()
+        pr.images_per_problem = int(images_per_problem)
+        pr.c_weight, pr.s_weight = c_weight.data_ptr(), s_weight.data_ptr()
+        self.problems = pr
 
     # ---- targets -------------------------------------------------------------------------
     def set_input_mask(self, mask: Optional[torch.Tensor]):
@@ -263,6 +283,11 @@ class NstEngine:
         _lib.call("isx_nst_backward", ctypes.byref(self.cfg), ctypes.byref(self.bufs), arr, lp, grad, _lib.stream_ptr())
 
     def eval(self, x: torch.Tensor, grad: torch.Tensor):
+        if self.problems is not None:
+            self.problems.style_target_b = self.cfg.style_target_b   # the batch of the targets set last
+            _lib.call("isx_nst_eval_problems", ctypes.byref(self.cfg), ctypes.byref(self.bufs), ctypes.byref(self.problems),
+                      x, self.loss_c, self.loss_s, grad, _lib.stream_ptr())
+            return
         _lib.call("isx_nst_eval", ctypes.byref(self.cfg), ctypes.byref(self.bufs), x, self.loss_c, self.loss_s, grad,
                   _lib.stream_ptr())
 

@@ -48,7 +48,11 @@ def stylize_frames(frames: torch.Tensor,
     (1,h,w) / (3,h,w) unbatched like …2020.py:103-104, or [B|1,1|3,h,w]; segs: label maps [B,1,H,W], host or device
     (int64 and uint8 are read as they are, uint8 moves 1 B per pixel; or `segmenter`, e.g. iris_b200.RITnet).  Returns (new_frames [B,1,H,W] on the device, info) with info = {masks, bboxes, valid, irises,
     c_loss_hist, s_loss_hist, evals, timings_ms}.  Frames without a single iris pixel are returned unchanged
-    (valid[i] False; the reference would fail in crop_image)."""
+    (valid[i] False; the reference would fail in crop_image).  nst()'s `problem_size` is not accepted: dropping the frames
+    without an iris would leave problems of unequal size."""
+    if "problem_size" in nst_kw:
+        raise ValueError("stylize_frames does not take problem_size: frames without an iris are dropped from the NST batch, "
+                         "so its problems would not all have the same size")
     dev = torch.device(device)
     if dev.type != 'cuda':
         raise _lib.IsxError("iris_b200.stylize_frames runs on a CUDA B200 only; there is no CPU path")

@@ -7,7 +7,9 @@ synchronisation except one flag read-back every `max_iter` evaluations."""
 from __future__ import annotations
 
 import ctypes
-from typing import List, Optional, Tuple
+import math
+import numbers
+from typing import List, Optional, Sequence, Tuple, Union
 
 import torch
 
@@ -44,13 +46,57 @@ def _norm_mask(mask: torch.Tensor, B: int, H: int, W: int, name: str, dev) -> to
     return m
 
 
+def _is_scalar(w) -> bool:
+    return isinstance(w, numbers.Real) or (torch.is_tensor(w) and w.dim() == 0)
+
+
+def _problem_layout(c_img, s_img, c_loss_weight, s_loss_weight, independent, problem_size, streams):
+    """Images per problem g of an nst() call, or None for the two layouts without per-problem weights (the whole batch
+    as one problem, or one problem per image with `independent`).  Checks everything on the host, before any device
+    work: B % g, the weight vector lengths (P = B / g), the style batch (1, P or B) and the option combinations."""
+    B = c_img.shape[0] if c_img.dim() == 4 else 1
+    vectors = not (_is_scalar(c_loss_weight) and _is_scalar(s_loss_weight))
+    if problem_size is None:
+        if not vectors:
+            return None
+        g = 1 if independent else B       # a weight vector with the default layouts: one weight per problem
+    else:
+        g = int(problem_size)
+        if g < 1 or g != problem_size or B % g:
+            raise ValueError("problem_size %r must divide the batch of %d images" % (problem_size, B))
+        if independent and g > 1:
+            raise ValueError("independent=True means problem_size=1, got problem_size=%d" % g)
+    P = B // g
+    for name, w in (("c_loss_weight", c_loss_weight), ("s_loss_weight", s_loss_weight)):
+        if not _is_scalar(w):
+            t = torch.as_tensor(w)
+            if t.dim() != 1 or t.numel() != P:
+                raise ValueError("%s must be a scalar or a 1-D sequence of %d weights (one per problem), got shape %s"
+                                 % (name, P, tuple(t.shape)))
+    Bs = s_img.shape[0] if s_img.dim() == 4 else 1
+    if Bs not in (1, P, B):
+        raise ValueError("style batch %d must be 1, %d (one per problem) or %d (one per image)" % (Bs, P, B))
+    if streams > 1 and g > 1:
+        raise ValueError("streams > 1 needs one problem per image; problem_size=%d couples %d images" % (g, g))
+    return g
+
+
+def _weight_vector(w, P: int, dev) -> torch.Tensor:
+    """alpha or beta as a device float64 [P] tensor (a scalar is the same weight for every problem)."""
+    if _is_scalar(w):
+        return torch.full((P,), float(w), device=dev, dtype=torch.float64)
+    return torch.as_tensor(w).detach().to(dev, torch.float64).reshape(P).contiguous()
+
+
 class NstJob:
     """Device-resident state of one nst() call: targets, L-BFGS buffers, the evaluation engine.
-    `tick()` = one closure evaluation (pipelines.py:80-101) + one L-BFGS iteration for the whole batch."""
+    `tick()` = one closure evaluation (pipelines.py:80-101) + one L-BFGS iteration for the whole batch.
+    problem_size g (validated by _problem_layout): B / g coupled problems with per-problem weights; None: one problem,
+    or one per image with `independent`, with scalar weights."""
 
     def __init__(self, c_img, s_img, vgg, dev, clone_content=True, BN_loss=True, c_loss_weight=1.0,
                  s_loss_weight=1.0, lr=1.0, epochs=200, independent=False, history_size=100, x_init=None,
-                 history_dtype=torch.float32, c_mask=None, s_mask=None, lbfgs_stream=None):
+                 history_dtype=torch.float32, c_mask=None, s_mask=None, lbfgs_stream=None, problem_size=None):
         c_img, c_unbatched = _prep_images(c_img, dev)
         # optional second stream for the L-BFGS passes of every tick (NstJobGroup: a low-priority stream, so that the
         # HBM-bound history passes of this sub-batch run beside the tensor-bound convolutions of another one)
@@ -70,6 +116,11 @@ class NstJob:
         cc, sc = vgg.content_convs, vgg.style_convs
         self.independent = independent
         self.epochs = int(epochs)
+        problems = problem_size is not None
+        P = B // problem_size if problems else (B if independent else 1)
+        if problems:   # the weights live on the device; the scalar weights of the configs are not read
+            self.c_w, self.s_w = _weight_vector(c_loss_weight, P, dev), _weight_vector(s_loss_weight, P, dev)
+            c_loss_weight = s_loss_weight = math.nan
 
         # ---- targets (pipelines.py:62-68) ----
         levels = [CONV_LEVEL[i] for i in sc]
@@ -82,6 +133,8 @@ class NstJob:
         eng = NstEngine(packed, B, H, W, xc, cc, sc, style_mode=1 if BN_loss else 0, c_weight=c_loss_weight,
                         s_weight=s_loss_weight, coupled=not independent, style_mask_b=cmask_b,
                         pred_unbatched=c_unbatched)
+        if problems:
+            eng.set_problems(B // P, self.c_w, self.s_w)
         if cmask_b:
             eng.set_style_masks(mask_pyramid(c_mask, levels))
         eng.forward(c_img)
@@ -91,7 +144,7 @@ class NstJob:
             eng.forward(s_img)
             s_feats = [eng.tap_view(i) for i in sc]   # consumed below, before the engine runs again
         else:
-            if Bs not in (1, B):
+            if Bs not in ((1, P, B) if problems else (1, B)):
                 raise ValueError("style batch %d must be 1 or %d" % (Bs, B))
             seng = NstEngine(packed, Bs, Hs, Ws, xs, cc, sc)
             seng.forward(s_img)
@@ -116,7 +169,7 @@ class NstJob:
         self.eng = eng
 
         # ---- optimiser (pipelines.py:59): torch.optim.LBFGS([x], lr) defaults ----
-        P = B if independent else 1
+        self.problems = problems
         self.P, self.ipp, self.N = P, B // P, self.x.numel() // P
         # one (y, s) pair per iteration, so a short job never needs all 100 slots
         hist = max(1, min(int(history_size), self.epochs + 20))
@@ -146,6 +199,11 @@ class NstJob:
         _lib.call("isx_clamp01", self.x, _lib.i64(self.x.numel()), _lib.stream_ptr())  # pipelines.py:82 (first closure)
 
     def _lbfgs(self):
+        if self.problems:
+            _lib.call("isx_lbfgs_tick_problems", self.x, self.grad, self.grad_prev, self.Sh, self.Yh, self.state, self.mats,
+                      self.scratch, self.eng.loss_c, self.eng.loss_s, self.ipp, self.P, _lib.i64(self.N),
+                      ctypes.byref(self.cfg), self.c_w, self.s_w, self.hist_c, self.hist_s, self.ticks, _lib.stream_ptr())
+            return
         _lib.call("isx_lbfgs_tick", self.x, self.grad, self.grad_prev, self.Sh, self.Yh, self.state, self.mats,
                   self.scratch, self.eng.loss_c, self.eng.loss_s, self.ipp, self.P, _lib.i64(self.N),
                   ctypes.byref(self.cfg), self.hist_c, self.hist_s, self.ticks, _lib.stream_ptr())
@@ -242,14 +300,17 @@ class NstJobGroup:
                 return m
             return m[lo:hi]
 
+        weights = {k: kw.pop(k) for k in ("c_loss_weight", "s_loss_weight") if k in kw}
+
         for i, st in enumerate(self.streams):
             lo, hi = bounds[i], bounds[i + 1]
             st.wait_stream(main)
             with torch.cuda.stream(st):
                 si = s_img[lo:hi] if s_batched else s_img
                 xi = x_init[lo:hi] if x_init is not None else None
+                wi = {k: w if _is_scalar(w) else w[lo:hi] for k, w in weights.items()}   # per-image weights follow their images
                 self.jobs.append(NstJob(c_img[lo:hi], si, vgg, dev, x_init=xi, c_mask=part(c_mask, lo, hi, True),
-                                        s_mask=part(s_mask, lo, hi, s_batched), lbfgs_stream=self.aux[i], **kw))
+                                        s_mask=part(s_mask, lo, hi, s_batched), lbfgs_stream=self.aux[i], **wi, **kw))
         self.max_ticks = self.jobs[0].max_ticks
         self.epochs = self.jobs[0].epochs
         self.P = B
@@ -404,8 +465,8 @@ def nst(c_img: torch.Tensor,
         s_img: torch.Tensor,
         clone_content: bool = True,
         BN_loss: bool = True,
-        c_loss_weight: float = 1,
-        s_loss_weight: float = 1,
+        c_loss_weight: Union[float, Sequence[float], torch.Tensor] = 1,
+        s_loss_weight: Union[float, Sequence[float], torch.Tensor] = 1,
         lr: float = 1,
         epochs: int = 200,
         vgg: torch.nn.Module = None,
@@ -422,6 +483,7 @@ def nst(c_img: torch.Tensor,
         cuda_graph: Optional[bool] = None,
         c_mask: Optional[torch.Tensor] = None,
         s_mask: Optional[torch.Tensor] = None,
+        problem_size: Optional[int] = None,
         ) -> tuple[torch.Tensor, list, list, list]:
     """Neural style transfer pipeline (pipelines.py:8-110).
 
@@ -429,6 +491,14 @@ def nst(c_img: torch.Tensor,
       independent   False: the batch is ONE L-BFGS problem exactly like the reference (shared history,
                     content loss averaged over the batch, SURVEY.md F6).  True: every image is its own
                     problem (== calling the reference once per image with B=1); this is what shards.
+      problem_size  g: the batch is B / g problems, images [p*g, (p+1)*g) forming problem p, each exactly the
+                    reference's nst() on those g images (content loss averaged over them, style loss summed, its own
+                    L-BFGS history and exit tests), all advancing in one device job.  c_loss_weight / s_loss_weight may
+                    then be sequences or 1-D tensors of P = B / g weights (a scalar = the same for every problem; a
+                    weight sequence without problem_size means one weight per problem of the default layout).  The
+                    style batch is 1 (shared), P (one per problem) or B (one per image).  problem_size=B is the
+                    default layout, problem_size=1 is independent=True; independent=True with problem_size > 1 and
+                    streams > 1 with problem_size > 1 raise ValueError.
       x_hist_stride keep every k-th evaluated image in x_hist (1 = reference behaviour, 0 = none).
       history_size  L-BFGS history (torch default 100).
       x_init        replaces torch.rand (pipelines.py:54) when clone_content is False.
@@ -448,7 +518,12 @@ def nst(c_img: torch.Tensor,
                     stored in bf16, halving the HBM traffic and footprint of the L-BFGS passes (opt-in).
     c_loss_hist / s_loss_hist hold one float per closure evaluation, aggregated over the batch the way
     the reference's batched losses are (content: mean over images, style: sum over images); per-image
-    values are left in `pipelines.last_info`."""
+    values are left in `pipelines.last_info`.  With several problems the histories are the mean (content) and the sum
+    (style) over problems, and last_info['c_loss_per_problem'] / ['s_loss_per_problem'] ([evals, P]) hold each
+    problem's own."""
+    problem_size = _problem_layout(c_img, s_img, c_loss_weight, s_loss_weight, independent, problem_size, streams)
+    if problem_size == 1:
+        independent = True
     dev = torch.device(device)
     if dev.type != 'cuda':
         raise _lib.IsxError("iris_b200.nst runs on a CUDA B200 only (device=%r); there is no CPU fallback" % (device,))
@@ -460,7 +535,8 @@ def nst(c_img: torch.Tensor,
     with torch.cuda.device(dev), torch.no_grad():
         kw = dict(clone_content=clone_content, BN_loss=BN_loss, c_loss_weight=c_loss_weight,
                   s_loss_weight=s_loss_weight, lr=lr, epochs=epochs, independent=independent,
-                  history_size=history_size, x_init=x_init, history_dtype=history_dtype, c_mask=c_mask, s_mask=s_mask)
+                  history_size=history_size, x_init=x_init, history_dtype=history_dtype, c_mask=c_mask, s_mask=s_mask,
+                  problem_size=problem_size)
         if streams > 1 and independent and c_img.dim() == 4 and c_img.shape[0] > 1:
             c_dev, _ = _prep_images(c_img, dev)
             s_dev = s_img.detach().to(dev, torch.float32)
@@ -511,11 +587,12 @@ def nst(c_img: torch.Tensor,
             x_hist = hist.finish((n_evals + x_hist_stride - 1) // x_hist_stride)
         if c_img.dim() == 3:          # unbatched content image: the reference returns (3,H,W) (pipelines.py:52,110)
             x = x[0]
-        c_loss_hist = (hc.mean(dim=1) if independent else hc[:, 0]).tolist()
-        s_loss_hist = (hs.sum(dim=1) if independent else hs[:, 0]).tolist()
+        per_problem = independent or problem_size is not None
+        c_loss_hist = (hc.mean(dim=1) if per_problem else hc[:, 0]).tolist()
+        s_loss_hist = (hs.sum(dim=1) if per_problem else hs[:, 0]).tolist()
         last_info.clear()
         last_info.update(ticks=job.ticks, evals=n_evals, evals_per_problem=evals, c_loss_per_image=hc,
-                         s_loss_per_image=hs, problems=job.P)
+                         s_loss_per_image=hs, c_loss_per_problem=hc, s_loss_per_problem=hs, problems=job.P)
     return x, x_hist, c_loss_hist, s_loss_hist
 
 
