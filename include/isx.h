@@ -309,6 +309,36 @@ typedef struct {
 int isx_nst_eval_problems(const isx_nst_config* cfg, const isx_nst_buffers* bufs, const isx_nst_problems* problems,
                           const float* x, double* loss_c, double* loss_s, float* grad, isx_stream stream);
 
+/* ---- coupled problems of unequal size in one batch (nst(problem_sizes=(g_0, ..., g_{P-1}))) ----------------------------
+ * Problem p is the images [first_image[p], first_image[p+1]): its content loss is the mean over its g_p images, its style
+ * loss the sum, and it has its own alpha / beta.  The offsets are a HOST array, checked on the host and passed to the
+ * kernels by value on every call: the library allocates nothing for them and a captured launch stays valid after the
+ * caller's array is gone.  The weights are device arrays read on every call, as in isx_nst_problems.
+ * L-BFGS memory: problem p owns the floats [first_image[p] * n, first_image[p+1] * n) of x / grad / grad_prev (n = floats
+ * per image) and the history block S / Y + (history+1) * first_image[p] * n of (history+1) * g_p * n elements, so S and Y
+ * are (history+1) * B * n elements each; with equal sizes this is the [P][history+1][N] layout of isx_lbfgs_tick.
+ * Scratch: isx_lbfgs_scratch_bytes(P, n * max_p g_p, history). */
+#define ISX_MAX_RANGED_PROBLEMS 1024
+typedef struct {
+  int32_t n_problems;                   /* P, 1 .. ISX_MAX_RANGED_PROBLEMS */
+  int32_t style_target_b;               /* 1, P or B: all images read target 0, problem p's images target p, image b
+                                           target b; replaces cfg->style_target_b (isx_lbfgs_tick_ranges ignores it) */
+  const int32_t* first_image;           /* host [P+1]: first_image[0] = 0 < first_image[1] < ... < first_image[P] = B */
+  const double* c_weight;               /* device [P]: alpha of each problem (cfg->c_weight is not read) */
+  const double* s_weight;               /* device [P]: beta of each problem (cfg->s_weight is not read) */
+} isx_nst_problem_ranges;
+/* isx_nst_eval for P problems of unequal size: same outputs as isx_nst_eval_problems.  With equal sizes g this is
+ * isx_nst_eval_problems with images_per_problem = g, bit for bit. */
+int isx_nst_eval_ranges(const isx_nst_config* cfg, const isx_nst_buffers* bufs, const isx_nst_problem_ranges* ranges,
+                        const float* x, double* loss_c, double* loss_s, float* grad, isx_stream stream);
+/* isx_lbfgs_tick_problems for P problems of unequal size over a batch of B images of n_img floats each (layout above);
+ * loss_c / loss_s double [B], hist_c / hist_s double [evaluations][P].  With equal sizes g this is
+ * isx_lbfgs_tick_problems with images_per_problem = g and N = g * n_img, bit for bit. */
+int isx_lbfgs_tick_ranges(float* x, const float* grad, float* grad_prev, void* S, void* Y, void* state, void* mats,
+                          void* scratch, const double* loss_c, const double* loss_s, const isx_nst_problem_ranges* ranges,
+                          int B, int64_t n_img, const isx_lbfgs_config* cfg, double* hist_c, double* hist_s, int tick,
+                          isx_stream stream);
+
 /* ---- K10: iris mask + bounding box (pipelines.py:139-165 mask_and_crop_iris; utils.py:44-72 crop_image) --
  * x fp32 [B,1,H,W]; seg int64 [B,1,H,W] label map or NULL; m = (seg == label) & (x <= threshold) (either
  * test can be off: seg NULL / use_threshold 0); mask uint8 [B,1,H,W] (0/1) and xm = x*m are optional

@@ -28,6 +28,8 @@ static constexpr int kDotThreads = 256;
 static constexpr int kElemsPerThread = 8;
 static constexpr int kChunk = kDotThreads * kElemsPerThread;  // elements per block
 
+__host__ __device__ __forceinline__ int nblk_of(long N) { return static_cast<int>((N + kChunk - 1) / kChunk); }
+
 __device__ __forceinline__ void load8(const float* p, long i, long n, float (&v)[8]) {
   if (i + 8 <= n && (reinterpret_cast<uintptr_t>(p + i) & 15) == 0) {
     const float4 a = __ldg(reinterpret_cast<const float4*>(p + i));
@@ -84,29 +86,47 @@ __device__ __forceinline__ float hround(float v, const __nv_bfloat16*) { return 
 // ---------------------------------------------------------------------------------------------
 // pass 1
 // partial layout: part[p][blk][slot][4] floats then extras: ext[p][blk][4] = {sum g^2, sum |g|, max |g|, 0}
+// kPerProblem: problem p owns the floats [vb, vb + N_p) of g / g_prev / x (vb = pr.vec_begin(p), N_p = pr.vec_size(p)) and
+// the history block S / Y + M1 * vb, slot k at k * N_p; the grid spans the largest problem (nblk blocks) and the blocks
+// past lbfgs_nblk(N_p) return at once, so a problem's block partition, and with it its summation order, depends on N_p only
 // ---------------------------------------------------------------------------------------------
-template <typename HT>
+template <typename HT, bool kPerProblem>
 __global__ void __launch_bounds__(kDotThreads)
 lbfgs_dots_kernel(const float* __restrict__ g, const float* __restrict__ g_prev, const HT* __restrict__ S,
                   HT* __restrict__ Y, const LbfgsState* __restrict__ states, long N, int M1, int nblk,
-                  float* __restrict__ part, float* __restrict__ ext) {
+                  float* __restrict__ part, float* __restrict__ ext,
+                  const __grid_constant__ ProblemArg<kPerProblem, ProblemRanges> pr) {
   const int p = blockIdx.y;
   const LbfgsState& st = states[p];
   if (st.done) return;
+  long vb;
+  if constexpr (kPerProblem) {
+    vb = pr.vec_begin(p);
+    N = pr.vec_size(p);
+    if (static_cast<int>(blockIdx.x) >= nblk_of(N)) return;
+  }
+  // history slot k of problem p
+  auto hist = [&](int k) -> long {
+    if constexpr (kPerProblem) return M1 * vb + k * N;
+    else return (static_cast<long>(p) * M1 + k) * N;
+  };
   extern __shared__ float sm[];  // [M1][8 warps][4]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long i0 = static_cast<long>(blockIdx.x) * kChunk + threadIdx.x * kElemsPerThread;
-  const float* gp = g + p * N;
+  const float* gp;
+  if constexpr (kPerProblem) gp = g + vb;
+  else gp = g + p * N;
   float gv[8], yv[8];
   load8(gp, i0, N, gv);
   const bool have_prev = st.n_iter >= 1;
   const int cand = st.cand_slot;
   if (have_prev) {
     float pv[8];
-    load8(g_prev + p * N, i0, N, pv);
+    if constexpr (kPerProblem) load8(g_prev + vb, i0, N, pv);
+    else load8(g_prev + p * N, i0, N, pv);
 #pragma unroll
     for (int j = 0; j < 8; ++j) yv[j] = hround(gv[j] - pv[j], Y);  // lbfgs.py:404
-    hstore8(Y + (static_cast<long>(p) * M1 + cand) * N, i0, N, yv);
+    hstore8(Y + hist(cand), i0, N, yv);
   } else {
 #pragma unroll
     for (int j = 0; j < 8; ++j) yv[j] = 0.f;
@@ -127,12 +147,12 @@ lbfgs_dots_kernel(const float* __restrict__ g, const float* __restrict__ g_prev,
   for (int k = 0; k < nlive; ++k) {
     const int slot = k < st.hist_count ? (st.hist_head + k) % M1 : cand;
     float sv[8], hv[8];
-    hload8(S + (static_cast<long>(p) * M1 + slot) * N, i0, N, sv);
+    hload8(S + hist(slot), i0, N, sv);
     if (slot == cand) {
 #pragma unroll
       for (int j = 0; j < 8; ++j) hv[j] = yv[j];
     } else {
-      hload8(Y + (static_cast<long>(p) * M1 + slot) * N, i0, N, hv);
+      hload8(Y + hist(slot), i0, N, hv);
     }
     float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f;
 #pragma unroll
@@ -167,13 +187,18 @@ lbfgs_dots_kernel(const float* __restrict__ g, const float* __restrict__ g_prev,
 // ---------------------------------------------------------------------------------------------
 // reduce the per-block partials: one block per (slot | extras, problem) -> dots[p][slot][4], dots[p][M1][0..2]
 // (kept out of the control kernel: with 375+ partial blocks per image the serial sum was its latency floor)
+// kPerProblem: problem p sums its own lbfgs_nblk(pr.vec_size(p)) partials; the rows stay nblk apart
 // ---------------------------------------------------------------------------------------------
+template <bool kPerProblem>
 __global__ void __launch_bounds__(128)
 lbfgs_reduce_kernel(const LbfgsState* __restrict__ states, const float* __restrict__ part,
-                    const float* __restrict__ ext, int M1, int nblk, double* __restrict__ dots) {
+                    const float* __restrict__ ext, int M1, int nblk, double* __restrict__ dots,
+                    const __grid_constant__ ProblemArg<kPerProblem, ProblemRanges> pr) {
   const int p = blockIdx.y;
   const LbfgsState& st = states[p];
   if (st.done) return;
+  int nb = nblk;   // partials of this problem
+  if constexpr (kPerProblem) nb = nblk_of(pr.vec_size(p));
   const int slot = blockIdx.x;
   __shared__ double red[4][4];
   double a0 = 0, a1 = 0, a2 = 0, a3 = 0;
@@ -182,12 +207,12 @@ lbfgs_reduce_kernel(const LbfgsState* __restrict__ states, const float* __restri
     // live ring slots and the candidate only
     const int rel = (slot - st.hist_head + M1) % M1;
     if (!(rel < st.hist_count || slot == st.cand_slot)) return;
-    for (int b = threadIdx.x; b < nblk; b += blockDim.x) {
+    for (int b = threadIdx.x; b < nb; b += blockDim.x) {
       const float4 q = __ldg(reinterpret_cast<const float4*>(part + ((static_cast<long>(p) * nblk + b) * M1 + slot) * 4));
       a0 += q.x; a1 += q.y; a2 += q.z; a3 += q.w;
     }
   } else {
-    for (int b = threadIdx.x; b < nblk; b += blockDim.x) {
+    for (int b = threadIdx.x; b < nb; b += blockDim.x) {
       const float4 q = __ldg(reinterpret_cast<const float4*>(ext + (static_cast<long>(p) * nblk + b) * 4));
       a0 += q.x; a1 += q.y; a2 = fmax(a2, static_cast<double>(q.z));
     }
@@ -220,14 +245,16 @@ __device__ __forceinline__ double block_sum_128(double v, double* red) {
   return red[0] + red[1] + red[2] + red[3];
 }
 
-// kPerProblem: the loss weights of problem p are c_w[p], s_w[p] (device arrays) instead of cfg.c_weight, cfg.s_weight
+// kPerProblem: the loss weights of problem p are c_w[p], s_w[p] (device arrays) instead of cfg.c_weight, cfg.s_weight, and
+// its losses are those of the images [pr.begin(p), pr.begin(p) + pr.size(p))
 template <bool kPerProblem>
 __global__ void __launch_bounds__(128)
 lbfgs_control_kernel(LbfgsState* __restrict__ states, double* __restrict__ mats, const double* __restrict__ dots,
                      const double* __restrict__ loss_c,
                      const double* __restrict__ loss_s, int images_per_problem, int M1, LbfgsConfig cfg,
                      double* __restrict__ hist_c, double* __restrict__ hist_s, int tick, int P,
-                     const double* __restrict__ c_w, const double* __restrict__ s_w) {
+                     const double* __restrict__ c_w, const double* __restrict__ s_w,
+                     const __grid_constant__ ProblemArg<kPerProblem, ProblemRanges> pr) {
   const int p = blockIdx.x;
   LbfgsState& st = states[p];
   __shared__ double red[4];
@@ -239,9 +266,17 @@ lbfgs_control_kernel(LbfgsState* __restrict__ states, double* __restrict__ mats,
 
   // ---- losses of this evaluation (logged like pipelines.py:94-95) ----
   double lc = 0.0, ls = 0.0;
-  for (int i = tid; i < images_per_problem; i += blockDim.x) {
-    lc += loss_c[p * images_per_problem + i];
-    ls += loss_s[p * images_per_problem + i];
+  if constexpr (kPerProblem) {
+    const int first = pr.begin(p), g = pr.size(p);
+    for (int i = tid; i < g; i += blockDim.x) {
+      lc += loss_c[first + i];
+      ls += loss_s[first + i];
+    }
+  } else {
+    for (int i = tid; i < images_per_problem; i += blockDim.x) {
+      lc += loss_c[p * images_per_problem + i];
+      ls += loss_s[p * images_per_problem + i];
+    }
   }
   lc = block_sum_128(lc, red);
   ls = block_sum_128(ls, red);
@@ -452,17 +487,32 @@ lbfgs_control_kernel(LbfgsState* __restrict__ states, double* __restrict__ mats,
 // ---------------------------------------------------------------------------------------------
 // pass 2
 // ---------------------------------------------------------------------------------------------
-template <typename HT>
+// kPerProblem: the slices of lbfgs_dots_kernel
+template <typename HT, bool kPerProblem>
 __global__ void __launch_bounds__(kDotThreads)
 lbfgs_update_kernel(float* __restrict__ x, const float* __restrict__ g, float* __restrict__ g_prev,
                     HT* __restrict__ S, const HT* __restrict__ Y, LbfgsState* __restrict__ states, long N,
-                    int M1) {
+                    int M1, const __grid_constant__ ProblemArg<kPerProblem, ProblemRanges> pr) {
   const int p = blockIdx.y;
   LbfgsState& st = states[p];
   if (!st.compute_d) return;
+  long vb;
+  if constexpr (kPerProblem) {
+    vb = pr.vec_begin(p);
+    N = pr.vec_size(p);
+    if (static_cast<int>(blockIdx.x) >= nblk_of(N)) return;
+  }
+  auto hist = [&](int k) -> long {
+    if constexpr (kPerProblem) return M1 * vb + k * N;
+    else return (static_cast<long>(p) * M1 + k) * N;
+  };
+  auto vec = [&]() -> long {
+    if constexpr (kPerProblem) return vb;
+    else return p * N;
+  };
   const long i0 = static_cast<long>(blockIdx.x) * kChunk + threadIdx.x * kElemsPerThread;
   float gv[8], d[8];
-  load8(g + p * N, i0, N, gv);
+  load8(g + vec(), i0, N, gv);
   const float cg = st.coef_g;
 #pragma unroll
   for (int j = 0; j < 8; ++j) d[j] = cg * gv[j];
@@ -471,8 +521,8 @@ lbfgs_update_kernel(float* __restrict__ x, const float* __restrict__ g, float* _
     const int slot = (head + k) % M1;
     const float a = st.coef_s[slot], b = st.coef_y[slot];
     float sv[8], yv[8];
-    hload8(S + (static_cast<long>(p) * M1 + slot) * N, i0, N, sv);
-    hload8(Y + (static_cast<long>(p) * M1 + slot) * N, i0, N, yv);
+    hload8(S + hist(slot), i0, N, sv);
+    hload8(Y + hist(slot), i0, N, yv);
 #pragma unroll
     for (int j = 0; j < 8; ++j) d[j] = fmaf(a, sv[j], fmaf(b, yv[j], d[j]));
   }
@@ -481,14 +531,14 @@ lbfgs_update_kernel(float* __restrict__ x, const float* __restrict__ g, float* _
   float mx = 0.f;
 #pragma unroll
   for (int j = 0; j < 8; ++j) { sv[j] = d[j] * t; mx = fmaxf(mx, fabsf(sv[j])); }  // s = d.mul(t), lbfgs.py:405
-  hstore8(S + (static_cast<long>(p) * M1 + st.cand_slot) * N, i0, N, sv);
-  store8(g_prev + p * N, i0, N, gv);  // lbfgs.py:444-447
+  hstore8(S + hist(st.cand_slot), i0, N, sv);
+  store8(g_prev + vec(), i0, N, gv);  // lbfgs.py:444-447
   if (st.apply) {
     float xv[8];
-    load8(x + p * N, i0, N, xv);
+    load8(x + vec(), i0, N, xv);
 #pragma unroll
     for (int j = 0; j < 8; ++j) xv[j] = fminf(fmaxf(fmaf(t, d[j], xv[j]), 0.f), 1.f);  // lbfgs.py:313 + pipelines.py:82
-    store8(x + p * N, i0, N, xv);
+    store8(x + vec(), i0, N, xv);
   }
   mx = warp_max(mx);
   if ((threadIdx.x & 31) == 0 && mx > 0.f) atomicMax(&st.max_td_bits, __float_as_uint(mx));
@@ -510,7 +560,7 @@ __global__ void lbfgs_init_kernel(LbfgsState* states, int P) {
   st.coef_g = 0.f;
 }
 
-int lbfgs_nblk(long N) { return static_cast<int>((N + kChunk - 1) / kChunk); }
+int lbfgs_nblk(long N) { return nblk_of(N); }
 
 int lbfgs_init(LbfgsState* states, int P, cudaStream_t s) {
   lbfgs_init_kernel<<<(P + 127) / 128, 128, 0, s>>>(states, P);
@@ -528,35 +578,54 @@ int clamp01(float* x, long n, cudaStream_t s) {
 int lbfgs_tick(float* x, const float* g, float* g_prev, void* S, void* Y, int history_bf16, LbfgsState* states, double* mats,
                float* part, float* ext, double* dots, const double* loss_c, const double* loss_s, int images_per_problem, int P,
                long N, const LbfgsConfig& cfg, double* hist_c, double* hist_s, int tick, cudaStream_t s, const double* c_w,
-               const double* s_w) {
+               const double* s_w, const ProblemRanges* pr) {
   const int M1 = cfg.history + 1;
   ISX_REQUIRE(M1 <= kMaxSlots, "lbfgs: history %d exceeds %d", cfg.history, kMaxSlots - 1);
   const int nblk = lbfgs_nblk(N);
   dim3 grid(nblk, P);
   const size_t sm1 = static_cast<size_t>(M1) * 8 * 4 * sizeof(float);
   isx_prof_begin(ISX_PROF_LBFGS, 0.0, s);  // both history passes + control; bytes are derived by the caller
-  if (history_bf16)
-    lbfgs_dots_kernel<__nv_bfloat16><<<grid, kDotThreads, sm1, s>>>(g, g_prev, static_cast<const __nv_bfloat16*>(S),
-                                                                    static_cast<__nv_bfloat16*>(Y), states, N, M1, nblk, part, ext);
-  else
-    lbfgs_dots_kernel<float><<<grid, kDotThreads, sm1, s>>>(g, g_prev, static_cast<const float*>(S), static_cast<float*>(Y),
-                                                            states, N, M1, nblk, part, ext);
-  ISX_LAUNCH_CHECK();
-  lbfgs_reduce_kernel<<<dim3(M1 + 1, P), 128, 0, s>>>(states, part, ext, M1, nblk, dots);
-  ISX_LAUNCH_CHECK();
-  if (c_w)
+  if (pr) {   // several problems with their own weights: grid over the largest problem (N), slices from the descriptor
+    if (history_bf16)
+      lbfgs_dots_kernel<__nv_bfloat16, true><<<grid, kDotThreads, sm1, s>>>(
+          g, g_prev, static_cast<const __nv_bfloat16*>(S), static_cast<__nv_bfloat16*>(Y), states, N, M1, nblk, part, ext, *pr);
+    else
+      lbfgs_dots_kernel<float, true><<<grid, kDotThreads, sm1, s>>>(g, g_prev, static_cast<const float*>(S),
+                                                                    static_cast<float*>(Y), states, N, M1, nblk, part, ext, *pr);
+    ISX_LAUNCH_CHECK();
+    lbfgs_reduce_kernel<true><<<dim3(M1 + 1, P), 128, 0, s>>>(states, part, ext, M1, nblk, dots, *pr);
+    ISX_LAUNCH_CHECK();
     lbfgs_control_kernel<true><<<P, 128, 0, s>>>(states, mats, dots, loss_c, loss_s, images_per_problem, M1, cfg, hist_c,
-                                                 hist_s, tick, P, c_w, s_w);
-  else
+                                                 hist_s, tick, P, c_w, s_w, *pr);
+    ISX_LAUNCH_CHECK();
+    if (history_bf16)
+      lbfgs_update_kernel<__nv_bfloat16, true><<<grid, kDotThreads, 0, s>>>(
+          x, g, g_prev, static_cast<__nv_bfloat16*>(S), static_cast<const __nv_bfloat16*>(Y), states, N, M1, *pr);
+    else
+      lbfgs_update_kernel<float, true><<<grid, kDotThreads, 0, s>>>(x, g, g_prev, static_cast<float*>(S),
+                                                                    static_cast<const float*>(Y), states, N, M1, *pr);
+  } else {
+    if (history_bf16)
+      lbfgs_dots_kernel<__nv_bfloat16, false><<<grid, kDotThreads, sm1, s>>>(
+          g, g_prev, static_cast<const __nv_bfloat16*>(S), static_cast<__nv_bfloat16*>(Y), states, N, M1, nblk, part, ext,
+          NoProblems());
+    else
+      lbfgs_dots_kernel<float, false><<<grid, kDotThreads, sm1, s>>>(g, g_prev, static_cast<const float*>(S),
+                                                                     static_cast<float*>(Y), states, N, M1, nblk, part, ext,
+                                                                     NoProblems());
+    ISX_LAUNCH_CHECK();
+    lbfgs_reduce_kernel<false><<<dim3(M1 + 1, P), 128, 0, s>>>(states, part, ext, M1, nblk, dots, NoProblems());
+    ISX_LAUNCH_CHECK();
     lbfgs_control_kernel<false><<<P, 128, 0, s>>>(states, mats, dots, loss_c, loss_s, images_per_problem, M1, cfg, hist_c,
-                                                  hist_s, tick, P, nullptr, nullptr);
-  ISX_LAUNCH_CHECK();
-  if (history_bf16)
-    lbfgs_update_kernel<__nv_bfloat16><<<grid, kDotThreads, 0, s>>>(x, g, g_prev, static_cast<__nv_bfloat16*>(S),
-                                                                    static_cast<const __nv_bfloat16*>(Y), states, N, M1);
-  else
-    lbfgs_update_kernel<float><<<grid, kDotThreads, 0, s>>>(x, g, g_prev, static_cast<float*>(S), static_cast<const float*>(Y),
-                                                            states, N, M1);
+                                                  hist_s, tick, P, nullptr, nullptr, NoProblems());
+    ISX_LAUNCH_CHECK();
+    if (history_bf16)
+      lbfgs_update_kernel<__nv_bfloat16, false><<<grid, kDotThreads, 0, s>>>(
+          x, g, g_prev, static_cast<__nv_bfloat16*>(S), static_cast<const __nv_bfloat16*>(Y), states, N, M1, NoProblems());
+    else
+      lbfgs_update_kernel<float, false><<<grid, kDotThreads, 0, s>>>(x, g, g_prev, static_cast<float*>(S),
+                                                                     static_cast<const float*>(Y), states, N, M1, NoProblems());
+  }
   isx_prof_end(ISX_PROF_LBFGS, s);
   ISX_LAUNCH_CHECK();
   return 0;

@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "isx_kernels.h"
+
 namespace isx {
 
 static constexpr int kMaxSlots = 104;  // history_size (<= 100, torch default) + 1 candidate slot, padded
@@ -43,6 +45,7 @@ int lbfgs_tick(float* x, const float* g, float* g_prev, void* S, void* Y, int hi
                double* mats,
                float* part, float* ext, double* dots, const double* loss_c, const double* loss_s, int images_per_problem, int P,
                long N, const LbfgsConfig& cfg, double* hist_c, double* hist_s, int tick, cudaStream_t s,
-               const double* c_w = nullptr, const double* s_w = nullptr);  // per-problem alpha / beta (device [P]) or cfg's
+               const double* c_w = nullptr, const double* s_w = nullptr,   // per-problem alpha / beta (device [P]) or cfg's
+               const ProblemRanges* pr = nullptr);   // with c_w: the problems' slices (N = floats of the largest problem)
 
 }  // namespace isx

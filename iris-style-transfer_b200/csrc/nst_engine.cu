@@ -1,6 +1,7 @@
 // Host-side driver of one NST closure evaluation (pipelines.py:80-91): VGG-19 forward to the deepest
 // tap, style/content losses, backward to the image -- a fixed sequence of libisx kernels on one
 // stream (graph-capturable: no allocation, no host synchronisation).  Also the L-BFGS C-ABI glue.
+#include <algorithm>
 #include <vector>
 
 #include "../../include/isx.h"
@@ -363,10 +364,38 @@ int run_backward(const isx_nst_config* c, const isx_nst_buffers* b, const Layout
 }  // namespace
 
 namespace {
-// One closure evaluation.  pr == nullptr: the batch is one problem (c->coupled) or B problems, with the scalar weights of
-// c.  Otherwise the batch is B / g problems of g images, each with its own alpha / beta (device arrays) and the style
-// target of image b at b / (B / pr->style_target_b); the arguments were validated by isx_nst_eval_problems.
-int nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_problems* pr, const float* x, double* loss_c,
+static_assert(kMaxRangedProblems == ISX_MAX_RANGED_PROBLEMS, "ProblemRanges holds the offsets of the largest layout");
+
+// Several problems of one evaluation, validated by isx_nst_eval_problems / isx_nst_eval_ranges
+struct ProblemSet {
+  ProblemRanges r;
+  int style_target_b;        // 1, P or B
+  const double* c_weight;    // device [P]
+  const double* s_weight;
+};
+
+// The checks isx_nst_eval_ranges and isx_lbfgs_tick_ranges share, before any device work: P within the limit, the offsets
+// 0 = first_image[0] < ... < first_image[P] = B, the weight arrays; copies the offsets into r.
+int load_ranges(const char* fn, const isx_nst_problem_ranges* pr, int B, ProblemRanges* r) {
+  ISX_REQUIRE(pr && pr->first_image, "%s: null pointer", fn);
+  const int P = pr->n_problems;
+  ISX_REQUIRE(P >= 1 && P <= ISX_MAX_RANGED_PROBLEMS, "%s: problem count %d must be in 1..%d", fn, P, ISX_MAX_RANGED_PROBLEMS);
+  ISX_REQUIRE(pr->first_image[0] == 0, "%s: first_image[0] = %d must be 0", fn, pr->first_image[0]);
+  for (int p = 0; p < P; ++p)
+    ISX_REQUIRE(pr->first_image[p + 1] > pr->first_image[p], "%s: first_image must increase strictly, problem %d is empty",
+                fn, p);
+  ISX_REQUIRE(pr->first_image[P] == B, "%s: first_image[%d] = %d must be the batch %d", fn, P, pr->first_image[P], B);
+  ISX_REQUIRE(pr->c_weight && pr->s_weight, "%s: null per-problem weight array", fn);
+  r->P = P;
+  r->ipp = 0;
+  for (int p = 0; p <= P; ++p) r->first[p] = pr->first_image[p];
+  return 0;
+}
+
+// One closure evaluation.  ps == nullptr: the batch is one problem (c->coupled) or B problems, with the scalar weights of
+// c.  Otherwise the batch is ps->r.P problems, each with its own alpha / beta (device arrays) and the style target of image
+// b at 0, its problem or b (style target batch 1, P or B).
+int nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const ProblemSet* ps, const float* x, double* loss_c,
              double* loss_s, float* grad, isx_stream stream) {
   Layout L;
   if (int rc = make_layout(c, &L)) return rc;
@@ -379,13 +408,15 @@ int nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_pr
   ISX_CHECK_CUDA(cudaMemsetAsync(loss_c, 0, sizeof(double) * B, s));
   ISX_CHECK_CUDA(cudaMemsetAsync(loss_s, 0, sizeof(double) * B, s));
   // per-problem beta of the style taps: the finalize kernels form beta_p * w * k2 (Gram) or beta_p * w / k2 (BN)
-  auto style_weights = [&](double w, double k2) {
-    ProblemWeights pw;
-    if (pr) {
-      pw.weight = pr->s_weight; pw.ipp = pr->images_per_problem; pw.target_div = B / pr->style_target_b;
-      pw.k1 = w; pw.k2 = k2;
-    }
-    return pw;
+  ProblemWeights pw;   // filled per tap below
+  if (ps) {
+    pw.r = ps->r;
+    pw.target = ps->style_target_b == B ? 2 : ps->style_target_b == 1 ? 0 : 1;
+  }
+  auto style_weights = [&](double w, double k2) -> const ProblemWeights* {
+    if (!ps) return nullptr;
+    pw.weight = ps->s_weight; pw.k1 = w; pw.k2 = k2;
+    return &pw;
   };
 
   // losses of everything tapped at `id` (a conv's ReLU output or a pool output), evaluated on the stored activation
@@ -410,10 +441,9 @@ int nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_pr
         const int splits = gram_pick_splits(B, static_cast<int>(HW), C);
         int rc = gram_sym_partial(act, B, static_cast<int>(HW), C, splits, atf(b, L.gram_ws), c->style_mask_b > 0 ? &gm : nullptr, s);
         if (rc) return rc;
-        const ProblemWeights pw = style_weights(w, inv_n);
         rc = gram_finalize(atf(b, L.gram_ws), B, splits, C, static_cast<float>(inv_n), nullptr, b->gram_target[st],
                            c->style_target_b, 0.25 * w, loss_s, static_cast<float>(c->s_weight * w * inv_n), at(b, L.D[st]), s,
-                           nullptr, 0, pr ? &pw : nullptr);
+                           nullptr, 0, style_weights(w, inv_n));
         if (rc) return rc;
       } else {  // StyleLoss_BN (utils.py:350-355)
         ISX_REQUIRE(b->bn_target_mean[st] && b->bn_target_std[st], "nst: BN target %d missing", st);
@@ -427,10 +457,9 @@ int nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_pr
         }
         int rc = chan_sums(act, B, HW, C, sums, s, m, c->style_mask_b);
         if (rc) return rc;
-        const ProblemWeights pw = style_weights(w, static_cast<double>(C));
         rc = bn_finalize(sums, B, C, HW, nullptr, nullptr, b->bn_target_mean[st], b->bn_target_std[st],
                          c->style_target_b, w / C, c->s_weight * w / C, loss_s, atf(b, L.aff_a[st]), atf(b, L.aff_b[st]), s,
-                         0, pr ? &pw : nullptr);
+                         0, style_weights(w, static_cast<double>(C)));
         if (rc) return rc;
         if (m)  // the gradient is no longer affine in F alone: m a + m^2 b F, materialised as a gradient map (buffer fm2)
           if (int rc2 = masked_affine_grad(act, m, c->style_mask_b, atf(b, L.aff_a[st]), atf(b, L.aff_b[st]), at(b, L.fm2[st]), B, HW, C, s)) return rc2;
@@ -440,13 +469,13 @@ int nst_eval(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_pr
     if (ct >= 0) {  // ContentLoss_L2 (utils.py:285-290): 0.5 * w * mean((p-t)^2)
       ISX_REQUIRE(b->content_target[ct], "nst: content target %d missing", ct);
       const long per_image = HW * C;
-      // F.mse_loss over the problem's batch: B images when coupled, g with several problems, else one
-      const double denom = static_cast<double>(per_image) * (pr ? pr->images_per_problem : c->coupled ? B : 1);
-      ProblemWeights pw;
-      if (pr) { pw.weight = pr->c_weight; pw.ipp = pr->images_per_problem; pw.k1 = c->content_w[ct]; pw.k2 = denom; }
+      // F.mse_loss over the problem's batch: B images when coupled, else one; with several problems the kernel forms
+      // per_image * g_p itself
+      const double denom = static_cast<double>(per_image) * (c->coupled ? B : 1);
+      if (ps) { pw.weight = ps->c_weight; pw.k1 = c->content_w[ct]; pw.k2 = static_cast<double>(per_image); }
       int rc = content_mse(act, reinterpret_cast<const bf16*>(b->content_target[ct]), c->content_target_b,
                            at(b, L.cgrad[ct]), B, per_image, 0.5 * c->content_w[ct] / denom,
-                           static_cast<float>(c->c_weight * c->content_w[ct] / denom), loss_c, s, 1, pr ? &pw : nullptr);
+                           static_cast<float>(c->c_weight * c->content_w[ct] / denom), loss_c, s, 1, ps ? &pw : nullptr);
       if (rc) return rc;
     }
     return 0;
@@ -508,9 +537,31 @@ extern "C" int isx_nst_eval_problems(const isx_nst_config* c, const isx_nst_buff
   ISX_REQUIRE(pr->c_weight && pr->s_weight, "isx_nst_eval_problems: null per-problem weight array");
   ISX_REQUIRE(c->style_mask_b == 0 || c->style_mask_b == 1 || c->style_mask_b == B,
               "isx_nst_eval_problems: style mask batch %d", c->style_mask_b);
-  isx_nst_problems q = *pr;
-  if (c->n_style == 0) q.style_target_b = B;   // no target is read
-  return nst_eval(c, b, &q, x, loss_c, loss_s, grad, stream);
+  ProblemSet ps;
+  ps.r.P = P;
+  ps.r.ipp = g;
+  ps.style_target_b = c->n_style == 0 ? B : tb;   // no target is read without style taps
+  ps.c_weight = pr->c_weight;
+  ps.s_weight = pr->s_weight;
+  return nst_eval(c, b, &ps, x, loss_c, loss_s, grad, stream);
+}
+
+extern "C" int isx_nst_eval_ranges(const isx_nst_config* c, const isx_nst_buffers* b, const isx_nst_problem_ranges* pr,
+                                   const float* x, double* loss_c, double* loss_s, float* grad, isx_stream stream) {
+  ISX_REQUIRE(c && b && pr && x && loss_c && loss_s && grad && b->workspace, "isx_nst_eval_ranges: null pointer");
+  ISX_REQUIRE(c->n_style + c->n_content > 0, "isx_nst_eval_ranges: no loss taps");
+  const int B = c->B;
+  ProblemSet ps;
+  if (int rc = load_ranges("isx_nst_eval_ranges", pr, B, &ps.r)) return rc;
+  const int P = ps.r.P, tb = pr->style_target_b;
+  ISX_REQUIRE(c->n_style == 0 || tb == 1 || tb == P || tb == B,
+              "isx_nst_eval_ranges: style target batch %d must be 1, %d (problems) or %d (images)", tb, P, B);
+  ISX_REQUIRE(c->style_mask_b == 0 || c->style_mask_b == 1 || c->style_mask_b == B,
+              "isx_nst_eval_ranges: style mask batch %d", c->style_mask_b);
+  ps.style_target_b = c->n_style == 0 ? B : tb;
+  ps.c_weight = pr->c_weight;
+  ps.s_weight = pr->s_weight;
+  return nst_eval(c, b, &ps, x, loss_c, loss_s, grad, stream);
 }
 
 extern "C" int isx_nst_prepare_style_masks(const isx_nst_config* c, const isx_nst_buffers* b, isx_stream stream) {
@@ -618,7 +669,7 @@ namespace {
 int lbfgs_tick_impl(float* x, const float* grad, float* grad_prev, void* Sh, void* Yh, void* state, void* mats, void* scratch,
                     const double* loss_c, const double* loss_s, int images_per_problem, int P, int64_t N,
                     const isx_lbfgs_config* cfg, const double* c_weight, const double* s_weight, double* hist_c,
-                    double* hist_s, int tick, isx_stream stream) {
+                    double* hist_s, int tick, isx_stream stream, const ProblemRanges* pr = nullptr) {
   LbfgsConfig lc;
   lc.epochs = cfg->epochs; lc.max_iter = cfg->max_iter; lc.max_eval = cfg->max_eval; lc.history = cfg->history;
   lc.lr = cfg->lr; lc.tolerance_grad = cfg->tolerance_grad; lc.tolerance_change = cfg->tolerance_change;
@@ -629,7 +680,7 @@ int lbfgs_tick_impl(float* x, const float* grad, float* grad_prev, void* Sh, voi
   const int64_t floats = static_cast<int64_t>(P) * nblk * (static_cast<int64_t>(cfg->history + 1) * 4 + 4);
   double* dots = reinterpret_cast<double*>(static_cast<char*>(scratch) + ((floats * 4 + 255) / 256) * 256);
   return lbfgs_tick(x, grad, grad_prev, Sh, Yh, cfg->history_bf16, static_cast<LbfgsState*>(state), static_cast<double*>(mats), part, ext,
-                    dots, loss_c, loss_s, images_per_problem, P, N, lc, hist_c, hist_s, tick, S(stream), c_weight, s_weight);
+                    dots, loss_c, loss_s, images_per_problem, P, N, lc, hist_c, hist_s, tick, S(stream), c_weight, s_weight, pr);
 }
 }  // namespace
 
@@ -656,8 +707,30 @@ extern "C" int isx_lbfgs_tick_problems(float* x, const float* grad, float* grad_
               P, images_per_problem, (long long)N);
   ISX_REQUIRE(cfg->history >= 1 && cfg->history <= 100, "isx_lbfgs_tick_problems: history %d must be in 1..100",
               cfg->history);
+  ProblemRanges r;
+  r.P = P;
+  r.ipp = images_per_problem;
+  r.n = N;
   return lbfgs_tick_impl(x, grad, grad_prev, Sh, Yh, state, mats, scratch, loss_c, loss_s, images_per_problem, P, N, cfg,
-                         c_weight, s_weight, hist_c, hist_s, tick, stream);
+                         c_weight, s_weight, hist_c, hist_s, tick, stream, &r);
+}
+
+extern "C" int isx_lbfgs_tick_ranges(float* x, const float* grad, float* grad_prev, void* Sh, void* Yh, void* state,
+                                     void* mats, void* scratch, const double* loss_c, const double* loss_s,
+                                     const isx_nst_problem_ranges* ranges, int B, int64_t n_img,
+                                     const isx_lbfgs_config* cfg, double* hist_c, double* hist_s, int tick,
+                                     isx_stream stream) {
+  ISX_REQUIRE(x && grad && grad_prev && Sh && Yh && state && mats && scratch && loss_c && loss_s && cfg && hist_c && hist_s,
+              "isx_lbfgs_tick_ranges: null pointer");
+  ProblemRanges r;
+  if (int rc = load_ranges("isx_lbfgs_tick_ranges", ranges, B, &r)) return rc;
+  ISX_REQUIRE(n_img >= 1, "isx_lbfgs_tick_ranges: %lld elements per image", (long long)n_img);
+  ISX_REQUIRE(cfg->history >= 1 && cfg->history <= 100, "isx_lbfgs_tick_ranges: history %d must be in 1..100", cfg->history);
+  r.n = n_img;
+  int g_max = 0;   // the grid of both history passes spans the largest problem
+  for (int p = 0; p < r.P; ++p) g_max = std::max(g_max, r.size(p));
+  return lbfgs_tick_impl(x, grad, grad_prev, Sh, Yh, state, mats, scratch, loss_c, loss_s, 0, r.P, g_max * n_img, cfg,
+                         ranges->c_weight, ranges->s_weight, hist_c, hist_s, tick, stream, &r);
 }
 
 __global__ void done_flags_kernel(const LbfgsState* st, int P, int32_t* out) {

@@ -90,6 +90,27 @@ class NstProblems(ctypes.Structure):
     ]
 
 
+class NstProblemRanges(ctypes.Structure):
+    _fields_ = [
+        ("n_problems", ctypes.c_int32), ("style_target_b", ctypes.c_int32),
+        ("first_image", ctypes.c_void_p), ("c_weight", ctypes.c_void_p), ("s_weight", ctypes.c_void_p),
+    ]
+
+
+def problem_ranges(first_image: Sequence[int], c_weight: torch.Tensor, s_weight: torch.Tensor):
+    """isx_nst_problem_ranges for the offsets first_image [P+1] (a host int32 array, returned with the struct: it must
+    outlive every call that reads the struct) and the device float64 [P] weights."""
+    P = len(first_image) - 1
+    for w in (c_weight, s_weight):
+        assert w.is_cuda and w.dtype == torch.float64 and w.is_contiguous() and w.shape == (P,)
+    offsets = (ctypes.c_int32 * (P + 1))(*[int(v) for v in first_image])
+    pr = NstProblemRanges()
+    pr.n_problems = P
+    pr.first_image = ctypes.cast(offsets, ctypes.c_void_p).value
+    pr.c_weight, pr.s_weight = c_weight.data_ptr(), s_weight.data_ptr()
+    return pr, offsets
+
+
 class PackedVGG:
     """VGG-19 conv parameters packed once for the device kernels (isx_pack_conv3x3_weights)."""
 
@@ -170,6 +191,7 @@ class NstEngine:
         self.loss_c = torch.zeros(B, device=self.device, dtype=torch.float64)
         self.loss_s = torch.zeros(B, device=self.device, dtype=torch.float64)
         self.problems: Optional[NstProblems] = None
+        self.ranges: Optional[NstProblemRanges] = None
 
     def set_problems(self, images_per_problem: int, c_weight: torch.Tensor, s_weight: torch.Tensor):
         """Evaluate the batch as B / images_per_problem coupled problems (isx_nst_eval_problems) with per-problem alpha /
@@ -182,6 +204,13 @@ class NstEngine:
         pr.images_per_problem = int(images_per_problem)
         pr.c_weight, pr.s_weight = c_weight.data_ptr(), s_weight.data_ptr()
         self.problems = pr
+
+    def set_problem_ranges(self, first_image: Sequence[int], c_weight: torch.Tensor, s_weight: torch.Tensor):
+        """Evaluate the batch as P coupled problems of unequal size (isx_nst_eval_ranges): problem p is the images
+        [first_image[p], first_image[p+1]), with per-problem alpha / beta as device float64 [P] tensors read on every
+        eval.  The offsets are checked by the library on every call."""
+        self.ranges, self._offsets = problem_ranges(first_image, c_weight, s_weight)
+        self._keep += [c_weight, s_weight]
 
     # ---- targets -------------------------------------------------------------------------
     def set_input_mask(self, mask: Optional[torch.Tensor]):
@@ -283,6 +312,11 @@ class NstEngine:
         _lib.call("isx_nst_backward", ctypes.byref(self.cfg), ctypes.byref(self.bufs), arr, lp, grad, _lib.stream_ptr())
 
     def eval(self, x: torch.Tensor, grad: torch.Tensor):
+        if self.ranges is not None:
+            self.ranges.style_target_b = self.cfg.style_target_b   # the batch of the targets set last
+            _lib.call("isx_nst_eval_ranges", ctypes.byref(self.cfg), ctypes.byref(self.bufs), ctypes.byref(self.ranges),
+                      x, self.loss_c, self.loss_s, grad, _lib.stream_ptr())
+            return
         if self.problems is not None:
             self.problems.style_target_b = self.cfg.style_target_b   # the batch of the targets set last
             _lib.call("isx_nst_eval_problems", ctypes.byref(self.cfg), ctypes.byref(self.bufs), ctypes.byref(self.problems),

@@ -13,12 +13,59 @@ bounding boxes.  The segmenter (the mask PRODUCER) is the caller's: pass its lab
 `segmenter(frames) -> label maps` such as iris_b200.RITnet (the 2019 driver's segmenter on the GPU)."""
 from __future__ import annotations
 
-from typing import Callable, Dict, Optional
+import numbers
+from typing import Callable, Dict, Optional, Sequence
 
 import torch
 
 from . import _lib
+from . import pipelines
 from .pipelines import composite_irises, crop_resize_irises, iris_masks_and_bboxes, nst
+
+
+def _batch(t) -> int:
+    return t.shape[0] if t.dim() == 4 else 1
+
+
+def frame_runs(B: int, frames_per_problem, style_batch: int, c_loss_weight=1, s_loss_weight=1) -> int:
+    """Number of runs K = ceil(B / g) of stylize_frames(frames_per_problem=g), after the host checks: g an integer >= 1,
+    each loss weight a scalar or K weights (one per run), the style batch 1, K or B."""
+    g = frames_per_problem
+    if isinstance(g, bool) or not isinstance(g, numbers.Integral) or g < 1:
+        raise ValueError("frames_per_problem must be an integer >= 1, got %r" % (g,))
+    K = (B + g - 1) // g
+    for name, w in (("c_loss_weight", c_loss_weight), ("s_loss_weight", s_loss_weight)):
+        if not pipelines._is_scalar(w):
+            t = torch.as_tensor(w)
+            if t.dim() != 1 or t.numel() != K:
+                raise ValueError("%s must be a scalar or a 1-D sequence of %d weights (one per run of %d frames), got "
+                                 "shape %s" % (name, K, g, tuple(t.shape)))
+    if style_batch not in (1, K, B):
+        raise ValueError("style batch %d must be 1, %d (one per run of %d frames) or %d (one per frame)"
+                         % (style_batch, K, g, B))
+    return K
+
+
+def group_frames(valid: Sequence[bool], frames_per_problem: int, style_batch: int = 1) -> Dict[str, object]:
+    """The NST layout of stylize_frames(frames_per_problem=g) from the per-frame iris flags: runs of g consecutive frames
+    (the last one may be shorter), each one coupled problem of the frames that have an iris.  Returns
+      run_sizes     [K] surviving frames per run (0: the run is skipped and all its frames come back unchanged)
+      kept_runs     the runs with at least one frame, one NST problem each; also the index map of per-run weights
+      problem_sizes their sizes (nst's problem_sizes)
+      frames        indices of the surviving frames (the NST batch, in order)
+      style_index   rows of the style batch the NST style images are taken from, or None for one shared style: the kept
+                    runs (style batch K) or the surviving frames (style batch B)"""
+    valid = [bool(v) for v in (valid.tolist() if torch.is_tensor(valid) else valid)]
+    B = len(valid)
+    K = frame_runs(B, frames_per_problem, style_batch)
+    g = int(frames_per_problem)
+    run_sizes = [sum(valid[k * g:(k + 1) * g]) for k in range(K)]
+    kept = [k for k in range(K) if run_sizes[k] > 0]
+    frames = [i for i in range(B) if valid[i]]
+    # with g = 1, K == B and both maps select the same rows
+    style_index = None if style_batch == 1 else frames if style_batch == B else kept
+    return dict(run_sizes=run_sizes, kept_runs=kept, problem_sizes=[run_sizes[k] for k in kept], frames=frames,
+                style_index=style_index)
 
 
 def _ev(dev):
@@ -43,16 +90,31 @@ def stylize_frames(frames: torch.Tensor,
                    device: str = 'cuda:0',
                    independent: bool = False,
                    inplace: bool = False,
+                   frames_per_problem: Optional[int] = None,
                    **nst_kw):
     """frames: [B,1,H,W] fp32 eye frames (host or device); style_iris: what the drivers hand to nst() as the style --
     (1,h,w) / (3,h,w) unbatched like …2020.py:103-104, or [B|1,1|3,h,w]; segs: label maps [B,1,H,W], host or device
     (int64 and uint8 are read as they are, uint8 moves 1 B per pixel; or `segmenter`, e.g. iris_b200.RITnet).  Returns (new_frames [B,1,H,W] on the device, info) with info = {masks, bboxes, valid, irises,
     c_loss_hist, s_loss_hist, evals, timings_ms}.  Frames without a single iris pixel are returned unchanged
     (valid[i] False; the reference would fail in crop_image).  nst()'s `problem_size` is not accepted: dropping the frames
-    without an iris would leave problems of unequal size."""
+    without an iris would leave problems of unequal size.
+
+    frames_per_problem=g: the frames form consecutive runs of g (the last one may be shorter), one driver batch each, and
+    every run is one coupled L-BFGS problem of its frames that have an iris -- the reference's nst() on that batch
+    (…2019.py:93-100, …2020.py:103-110) -- all in one device job (nst(problem_sizes=...)).  A run without any iris is
+    skipped.  c_loss_weight / s_loss_weight are scalars or K = ceil(B / g) weights (one per run); style_iris has batch 1,
+    K (one per run) or B (one per frame).  info then also holds problem_sizes (surviving frames per run, 0 for a skipped
+    run), evals_per_run ([K], 0 for a skipped run) and c_loss_per_run / s_loss_per_run ([evals, K], NaN for a skipped
+    run); c_loss_hist / s_loss_hist are the mean / sum over the problems that ran (see group_frames)."""
     if "problem_size" in nst_kw:
         raise ValueError("stylize_frames does not take problem_size: frames without an iris are dropped from the NST batch, "
                          "so its problems would not all have the same size")
+    if frames_per_problem is not None:
+        if independent:
+            raise ValueError("frames_per_problem couples the frames of each run; it cannot be combined with independent=True")
+        if "problem_sizes" in nst_kw:
+            raise ValueError("stylize_frames derives problem_sizes from frames_per_problem and the iris flags")
+        frame_runs(frames.shape[0], frames_per_problem, _batch(style_iris), c_loss_weight, s_loss_weight)
     dev = torch.device(device)
     if dev.type != 'cuda':
         raise _lib.IsxError("iris_b200.stylize_frames runs on a CUDA B200 only; there is no CPU path")
@@ -79,13 +141,28 @@ def stylize_frames(frames: torch.Tensor,
         valid_h = valid.cpu()                      # the one host synchronisation: which frames have an iris at all
         idx = torch.nonzero(valid_h).flatten()
         info: Dict[str, object] = dict(masks=masks, bboxes=bboxes, valid=valid_h)
+        runs = None
+        if frames_per_problem is not None:
+            runs = group_frames(valid_h, frames_per_problem, _batch(style_iris))
+            info.update(problem_sizes=runs["run_sizes"])
         if idx.numel() == 0:
             info.update(irises=crops, c_loss_hist=[], s_loss_hist=[], evals=0, timings_ms={})
+            if runs is not None:
+                K = len(runs["run_sizes"])
+                info.update(evals_per_run=[0] * K, c_loss_per_run=torch.full((0, K), float("nan"), dtype=torch.float64),
+                            s_loss_per_run=torch.full((0, K), float("nan"), dtype=torch.float64))
             return x, info
         all_valid = idx.numel() == B
         c_in = crops if all_valid else crops[idx.to(dev)]
         s_in = style_iris
-        if s_in.dim() == 4 and s_in.shape[0] == B and not all_valid:
+        if runs is not None:
+            if runs["style_index"] is not None:
+                s_in = s_in[torch.tensor(runs["style_index"], device=s_in.device)]
+            kept = runs["kept_runs"]
+            c_loss_weight, s_loss_weight = [w if pipelines._is_scalar(w) else torch.as_tensor(w).reshape(-1)[kept]
+                                            for w in (c_loss_weight, s_loss_weight)]
+            nst_kw["problem_sizes"] = runs["problem_sizes"]
+        elif s_in.dim() == 4 and s_in.shape[0] == B and not all_valid:
             s_in = s_in[idx.to(s_in.device)]
         if s_in.dim() == 4 and s_in.shape[1] == 1:
             s_in = s_in.repeat(1, 3, 1, 1)          # …2019.py:94 `s_irises.repeat(1, 3, 1, 1)`
@@ -101,6 +178,17 @@ def stylize_frames(frames: torch.Tensor,
             x[idx.to(dev)] = sub
         t5 = _ev(dev)
         torch.cuda.current_stream(dev).synchronize()
+        if runs is not None:
+            K, kept = len(runs["run_sizes"]), runs["kept_runs"]
+            lp = pipelines.last_info
+            ev = torch.zeros(K, dtype=torch.int64)
+            ev[kept] = lp["evals_per_problem"].to(torch.int64)
+            per_run = []
+            for h in (lp["c_loss_per_problem"], lp["s_loss_per_problem"]):
+                full = torch.full((h.shape[0], K), float("nan"), dtype=torch.float64)
+                full[:, kept] = h.to(torch.float64)
+                per_run.append(full)
+            info.update(evals_per_run=ev.tolist(), c_loss_per_run=per_run[0], s_loss_per_run=per_run[1])
         info.update(irises=new, c_loss_hist=c_hist, s_loss_hist=s_hist, evals=len(s_hist),
                     timings_ms=dict(upload_segment=t0.elapsed_time(t1), mask_bbox=t1.elapsed_time(t2),
                                     crop_resize=t2.elapsed_time(t3), nst=t3.elapsed_time(t4), composite=t4.elapsed_time(t5)))

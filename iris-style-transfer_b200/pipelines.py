@@ -81,6 +81,37 @@ def _problem_layout(c_img, s_img, c_loss_weight, s_loss_weight, independent, pro
     return g
 
 
+def _ranged_layout(c_img, s_img, c_loss_weight, s_loss_weight, independent, problem_size, problem_sizes, streams):
+    """The problem sizes (g_0, ..., g_{P-1}) of an nst(problem_sizes=...) call as a list of ints.  Checks everything on the
+    host, before any device work: every g_p an integer >= 1, their sum B, the weight vector lengths (P), the style batch
+    (1, P or B) and the options that cannot be combined with it."""
+    B = c_img.shape[0] if c_img.dim() == 4 else 1
+    if problem_size is not None:
+        raise ValueError("pass problem_size (equal problems) or problem_sizes, not both")
+    if independent:
+        raise ValueError("independent=True is problem_sizes=[1] * B; it cannot be combined with problem_sizes")
+    if streams > 1:
+        raise ValueError("streams > 1 needs one problem per image; it cannot be combined with problem_sizes")
+    sizes = list(problem_sizes.tolist() if torch.is_tensor(problem_sizes) else problem_sizes)
+    for g in sizes:
+        if isinstance(g, bool) or not isinstance(g, numbers.Integral) or g < 1:
+            raise ValueError("problem_sizes must be integers >= 1, got %r" % (sizes,))
+    sizes = [int(g) for g in sizes]
+    if sum(sizes) != B:
+        raise ValueError("problem_sizes %r sum to %d, not to the batch of %d images" % (sizes, sum(sizes), B))
+    P = len(sizes)
+    for name, w in (("c_loss_weight", c_loss_weight), ("s_loss_weight", s_loss_weight)):
+        if not _is_scalar(w):
+            t = torch.as_tensor(w)
+            if t.dim() != 1 or t.numel() != P:
+                raise ValueError("%s must be a scalar or a 1-D sequence of %d weights (one per problem), got shape %s"
+                                 % (name, P, tuple(t.shape)))
+    Bs = s_img.shape[0] if s_img.dim() == 4 else 1
+    if Bs not in (1, P, B):
+        raise ValueError("style batch %d must be 1, %d (one per problem) or %d (one per image)" % (Bs, P, B))
+    return sizes
+
+
 def _weight_vector(w, P: int, dev) -> torch.Tensor:
     """alpha or beta as a device float64 [P] tensor (a scalar is the same weight for every problem)."""
     if _is_scalar(w):
@@ -92,11 +123,13 @@ class NstJob:
     """Device-resident state of one nst() call: targets, L-BFGS buffers, the evaluation engine.
     `tick()` = one closure evaluation (pipelines.py:80-101) + one L-BFGS iteration for the whole batch.
     problem_size g (validated by _problem_layout): B / g coupled problems with per-problem weights; None: one problem,
-    or one per image with `independent`, with scalar weights."""
+    or one per image with `independent`, with scalar weights.  problem_sizes (validated by _ranged_layout): problems of
+    those sizes, one after the other, with per-problem weights."""
 
     def __init__(self, c_img, s_img, vgg, dev, clone_content=True, BN_loss=True, c_loss_weight=1.0,
                  s_loss_weight=1.0, lr=1.0, epochs=200, independent=False, history_size=100, x_init=None,
-                 history_dtype=torch.float32, c_mask=None, s_mask=None, lbfgs_stream=None, problem_size=None):
+                 history_dtype=torch.float32, c_mask=None, s_mask=None, lbfgs_stream=None, problem_size=None,
+                 problem_sizes=None):
         c_img, c_unbatched = _prep_images(c_img, dev)
         # optional second stream for the L-BFGS passes of every tick (NstJobGroup: a low-priority stream, so that the
         # HBM-bound history passes of this sub-batch run beside the tensor-bound convolutions of another one)
@@ -116,8 +149,9 @@ class NstJob:
         cc, sc = vgg.content_convs, vgg.style_convs
         self.independent = independent
         self.epochs = int(epochs)
-        problems = problem_size is not None
-        P = B // problem_size if problems else (B if independent else 1)
+        ranged = problem_sizes is not None
+        problems = problem_size is not None or ranged
+        P = len(problem_sizes) if ranged else B // problem_size if problems else (B if independent else 1)
         if problems:   # the weights live on the device; the scalar weights of the configs are not read
             self.c_w, self.s_w = _weight_vector(c_loss_weight, P, dev), _weight_vector(s_loss_weight, P, dev)
             c_loss_weight = s_loss_weight = math.nan
@@ -133,7 +167,9 @@ class NstJob:
         eng = NstEngine(packed, B, H, W, xc, cc, sc, style_mode=1 if BN_loss else 0, c_weight=c_loss_weight,
                         s_weight=s_loss_weight, coupled=not independent, style_mask_b=cmask_b,
                         pred_unbatched=c_unbatched)
-        if problems:
+        if ranged:
+            eng.set_problem_ranges([sum(problem_sizes[:p]) for p in range(P + 1)], self.c_w, self.s_w)
+        elif problems:
             eng.set_problems(B // P, self.c_w, self.s_w)
         if cmask_b:
             eng.set_style_masks(mask_pyramid(c_mask, levels))
@@ -169,8 +205,10 @@ class NstJob:
         self.eng = eng
 
         # ---- optimiser (pipelines.py:59): torch.optim.LBFGS([x], lr) defaults ----
-        self.problems = problems
-        self.P, self.ipp, self.N = P, B // P, self.x.numel() // P
+        self.problems, self.ranged = problems, ranged
+        self.n_img = xc * H * W
+        # N: floats of the largest problem (the grid and the scratch of the L-BFGS passes)
+        self.P, self.ipp, self.N = P, B // P, (max(problem_sizes) * self.n_img if ranged else self.x.numel() // P)
         # one (y, s) pair per iteration, so a short job never needs all 100 slots
         hist = max(1, min(int(history_size), self.epochs + 20))
         if history_dtype not in (torch.float32, torch.bfloat16):
@@ -186,8 +224,12 @@ class NstJob:
         self.mats = torch.zeros(_lib.call_i64("isx_lbfgs_mats_bytes", P, hist), device=dev, dtype=torch.uint8)
         self.scratch = torch.empty(_lib.call_i64("isx_lbfgs_scratch_bytes", P, _lib.i64(N), hist), device=dev,
                                    dtype=torch.uint8)
-        self.Sh = torch.empty(P, M1, N, device=dev, dtype=history_dtype)
-        self.Yh = torch.empty(P, M1, N, device=dev, dtype=history_dtype)
+        if ranged:   # problem p's block starts at M1 * first_p * n_img: with equal sizes the (P, M1, N) layout below
+            self.Sh = torch.empty(M1 * B * self.n_img, device=dev, dtype=history_dtype)
+            self.Yh = torch.empty(M1 * B * self.n_img, device=dev, dtype=history_dtype)
+        else:
+            self.Sh = torch.empty(P, M1, N, device=dev, dtype=history_dtype)
+            self.Yh = torch.empty(P, M1, N, device=dev, dtype=history_dtype)
         self.grad = torch.empty_like(self.x)
         self.grad_prev = torch.empty_like(self.x)
         self.hist_c = torch.zeros(self.max_ticks, P, device=dev, dtype=torch.float64)
@@ -199,6 +241,12 @@ class NstJob:
         _lib.call("isx_clamp01", self.x, _lib.i64(self.x.numel()), _lib.stream_ptr())  # pipelines.py:82 (first closure)
 
     def _lbfgs(self):
+        if self.ranged:
+            _lib.call("isx_lbfgs_tick_ranges", self.x, self.grad, self.grad_prev, self.Sh, self.Yh, self.state, self.mats,
+                      self.scratch, self.eng.loss_c, self.eng.loss_s, ctypes.byref(self.eng.ranges), self.x.shape[0],
+                      _lib.i64(self.n_img), ctypes.byref(self.cfg), self.hist_c, self.hist_s, self.ticks,
+                      _lib.stream_ptr())
+            return
         if self.problems:
             _lib.call("isx_lbfgs_tick_problems", self.x, self.grad, self.grad_prev, self.Sh, self.Yh, self.state, self.mats,
                       self.scratch, self.eng.loss_c, self.eng.loss_s, self.ipp, self.P, _lib.i64(self.N),
@@ -484,6 +532,7 @@ def nst(c_img: torch.Tensor,
         c_mask: Optional[torch.Tensor] = None,
         s_mask: Optional[torch.Tensor] = None,
         problem_size: Optional[int] = None,
+        problem_sizes: Optional[Sequence[int]] = None,
         ) -> tuple[torch.Tensor, list, list, list]:
     """Neural style transfer pipeline (pipelines.py:8-110).
 
@@ -499,6 +548,11 @@ def nst(c_img: torch.Tensor,
                     style batch is 1 (shared), P (one per problem) or B (one per image).  problem_size=B is the
                     default layout, problem_size=1 is independent=True; independent=True with problem_size > 1 and
                     streams > 1 with problem_size > 1 raise ValueError.
+      problem_sizes (g_0, ..., g_{P-1}), integers >= 1 summing to B: problems of unequal size, problem p being the images
+                    [g_0 + ... + g_{p-1}, g_0 + ... + g_p), each exactly the reference's nst() on its images, like
+                    problem_size (weights, style batch 1 / P / B and outputs as there).  [g] * P is problem_size=g, [B]
+                    the default layout and [1] * B independent=True, bit for bit.  It cannot be combined with
+                    problem_size, independent=True or streams > 1 (ValueError).
       x_hist_stride keep every k-th evaluated image in x_hist (1 = reference behaviour, 0 = none).
       history_size  L-BFGS history (torch default 100).
       x_init        replaces torch.rand (pipelines.py:54) when clone_content is False.
@@ -521,7 +575,11 @@ def nst(c_img: torch.Tensor,
     values are left in `pipelines.last_info`.  With several problems the histories are the mean (content) and the sum
     (style) over problems, and last_info['c_loss_per_problem'] / ['s_loss_per_problem'] ([evals, P]) hold each
     problem's own."""
-    problem_size = _problem_layout(c_img, s_img, c_loss_weight, s_loss_weight, independent, problem_size, streams)
+    if problem_sizes is not None:
+        problem_sizes = _ranged_layout(c_img, s_img, c_loss_weight, s_loss_weight, independent, problem_size,
+                                       problem_sizes, streams)
+    else:
+        problem_size = _problem_layout(c_img, s_img, c_loss_weight, s_loss_weight, independent, problem_size, streams)
     if problem_size == 1:
         independent = True
     dev = torch.device(device)
@@ -536,7 +594,7 @@ def nst(c_img: torch.Tensor,
         kw = dict(clone_content=clone_content, BN_loss=BN_loss, c_loss_weight=c_loss_weight,
                   s_loss_weight=s_loss_weight, lr=lr, epochs=epochs, independent=independent,
                   history_size=history_size, x_init=x_init, history_dtype=history_dtype, c_mask=c_mask, s_mask=s_mask,
-                  problem_size=problem_size)
+                  problem_size=problem_size, problem_sizes=problem_sizes)
         if streams > 1 and independent and c_img.dim() == 4 and c_img.shape[0] > 1:
             c_dev, _ = _prep_images(c_img, dev)
             s_dev = s_img.detach().to(dev, torch.float32)
@@ -587,7 +645,7 @@ def nst(c_img: torch.Tensor,
             x_hist = hist.finish((n_evals + x_hist_stride - 1) // x_hist_stride)
         if c_img.dim() == 3:          # unbatched content image: the reference returns (3,H,W) (pipelines.py:52,110)
             x = x[0]
-        per_problem = independent or problem_size is not None
+        per_problem = independent or problem_size is not None or problem_sizes is not None
         c_loss_hist = (hc.mean(dim=1) if per_problem else hc[:, 0]).tolist()
         s_loss_hist = (hs.sum(dim=1) if per_problem else hs[:, 0]).tolist()
         last_info.clear()
